@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the decombine hot path on B200 (driver contract: one JSON line on stdout from rank 0).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--reads R] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--reads R] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): synthetic 10 M x 250-nt reads, human beta, extended tag set,
 -br R2 -bl 42 -ol M13.  One "step" = one pass of the decombine kernels over the whole batch of packed
@@ -20,6 +20,7 @@ reads.  Weak scaling: every GPU gets its own 10 M-read shard of the same determi
 installed offline; its algorithm is what oracle/dcr_oracle.c restates and pins against reference fixtures).
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -58,7 +59,33 @@ def parse_args():
     ap.add_argument("--sub-rate", type=float, default=0.0, help="per-base substitution rate of the synthetic reads (default: the headline workload, 0)")
     ap.add_argument("--n-rate", type=float, default=0.0, help="per-base N rate")
     ap.add_argument("--no-workloads", action="store_true", help="skip the extra workload blocks (configs[2])")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's results of the last resident step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the CUDA path; --impl reference has none")
+    return args
+
+
+DUMP_READS = 1 << 20     # 10 record fields as float32 + the index as float64: 48 MiB of the 64 MB a dump may take
+
+
+def dump_outputs(dirname, res, cnt):
+    """What a caller of the resident path receives (the counters and every field of the result records), as .npy files
+    that two builds can be compared by: the records of a fixed, seeded sample of DUMP_READS reads (all reads when there
+    are no more), their read indices in read_index.npy."""
+    os.makedirs(dirname, exist_ok=True)
+    n = len(res)
+    if n > DUMP_READS:
+        idx = np.sort(np.random.default_rng(SEED).choice(n, DUMP_READS, replace=False))
+    else:
+        idx = np.arange(n)
+    np.save(os.path.join(dirname, "read_index.npy"), idx.astype(np.float64))
+    for f in res.dtype.names:
+        np.save(os.path.join(dirname, f + ".npy"), res[f][idx].astype(np.float32))
+    np.save(os.path.join(dirname, "counters.npy"), cnt.astype(np.float64))
 
 
 def make_reads(info, first, n, threads, sub_rate=0.0, n_rate=0.0):
@@ -110,7 +137,7 @@ def run_mixed(args, rank, world, local_rank, host_threads, stream, barrier, spec
     ln = np.full(n, READ_LEN, dtype=np.uint32)
     packed = _lib.pack_arrays(r1, off, ln, revcomp=True, n_threads=host_threads)
     del r1
-    steps = max(1, min(args.steps, 20))
+    steps = args.steps
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -195,7 +222,7 @@ def run_cfg3(args, rank, world, local_rank, host_threads, stream, barrier):
     ln = np.full(n, READ_LEN, dtype=np.uint32)
     packed = _lib.pack_arrays(r1, off, ln, revcomp=True, n_threads=host_threads)
     del r1
-    steps = max(1, min(args.steps, 20))
+    steps = args.steps
     vt, jt = info.tables()
     ctx = _lib.Context(vt, jt, device=local_rank)
     ctx.set_stream(stream.cuda_stream)
@@ -289,6 +316,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(index), "--query-gpu=" + self.FIELDS,
                                           "--format=csv,noheader,nounits", "-lms", "100"], stdout=subprocess.PIPE,
                                          stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)   # the sampler loops until killed: never outlive a run that fails before stop()
             self.t = threading.Thread(target=self._pump, daemon=True)
             self.t.start()
         except Exception:
@@ -426,6 +454,8 @@ def main():
         ms_total = ev0.elapsed_time(ev1)
         kms, klaunch = ctx.timing_get()
         ctx.timing_enable(False)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, *ctx.download())
         clocks = sampler.stop(t_spin + 0.1, t1) if sampler else None   # samples under load: spin-up (same kernels) + timed region
 
         # ---- e2e_packed: host packed buffers -> results in host memory through dcb_decombine_batch ----
@@ -433,7 +463,7 @@ def main():
             ctx.decombine(packed, pinned=True)
         barrier()
         e0 = time.perf_counter()
-        e2e_steps = max(1, min(args.steps, 10))
+        e2e_steps = args.steps
         for _ in range(e2e_steps):
             res_e, cnt_e = ctx.decombine(packed, pinned=True)   # synchronous: results are in host memory on return
         ep_ms = (time.perf_counter() - e0) * 1e3
