@@ -687,9 +687,20 @@ dcb_exact_kernel_flat(BatchDev b, QTables qt, DcrParams prm, int both_frames, dc
 // the 32-base window, more than DCB_HALF_CAP candidates) goes on to the general kernel through a second queue, uncounted.
 // Tables: 0 = V tag records, 1 = J tag records, 2 = half-tag index.
 // ------------------------------------------------------------------------------------------------
-#define DCB_HALF_CAP 12
+// The three capacities can be set at compile time (-D...): the test suite builds variants with tiny lists, in which nearly
+// every warp overflows every list, to run the pass-on branches on ordinary data (build.py variant, VARIANTS).
+#ifndef DCB_HALF_CAP
+#define DCB_HALF_CAP 12         // candidates of one read
+#endif
+#ifndef DCB_HALF_WCAP
 #define DCB_HALF_WCAP 192       // probe hits of one warp's 32 reads that are confirmed here; reads beyond pass on
-#define DCB_HALF_WCAP2 126      // (occurrence, tag) pairs of one warp's 32 reads
+#endif
+#ifndef DCB_HALF_WCAP2
+#define DCB_HALF_WCAP2 126      // prefix hits, and (occurrence, tag) pairs, of one warp's 32 reads
+#endif
+static_assert(DCB_HALF_WCAP % 2 == 0, "s_work holds 16-bit entries and is carved in 32-bit words");
+static_assert(DCB_HALF_WCAP2 >= 3, "a J-scan round takes reads until WCAP2 / 3 prefix hits");
+static_assert(DCB_HALF_CAP >= 1 && DCB_HALF_CAP <= 4095, "the candidate count of DCB_HALF_COUNT has 12 bits");
 template <int NW, int T>
 __global__ void __launch_bounds__(T, 1)
 dcb_halftag_kernel(BatchDev b, Tables4 tb, DcrParams prm, dcb_result* __restrict__ results,

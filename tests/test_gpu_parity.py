@@ -40,7 +40,9 @@ def test_cuda_matches_reference_fixtures(dcr_cases, force_general):
         packed.free(); ctx.close()
 
 
-@pytest.mark.parametrize("species,tagset,chain,orientation,L,sub,nrate,junk", [
+# (species, tag set, chain, orientation, read length, substitution, N and junk rates); test_gpu_halftag_capacity.py runs
+# them again on libraries built with the half-tag kernel's work lists shrunk
+SYNTHETIC_SHAPES = [
     ("human", "extended", "b", "reverse", 250, 0.0, 0.0, 0.0),       # BASELINE configs[1] shape
     ("human", "extended", "b", "reverse", 250, 0.01, 0.001, 0.05),   # configs[2] shape (beta half)
     ("human", "extended", "a", "reverse", 250, 0.01, 0.001, 0.05),   # configs[2] shape (alpha half)
@@ -53,7 +55,10 @@ def test_cuda_matches_reference_fixtures(dcr_cases, force_general):
     ("mouse", "original", "d", "both", 250, 0.005, 0.001, 0.02),
     ("mouse", "original", "a", "reverse", 250, 0.01, 0.001, 0.02),
     ("human", "original", "a", "reverse", 250, 0.01, 0.002, 0.02),   # flat kernel + N + 6-base J halves: the J scan over the invalid-base column
-])
+]
+
+
+@pytest.mark.parametrize("species,tagset,chain,orientation,L,sub,nrate,junk", SYNTHETIC_SHAPES)
 def test_cuda_matches_oracle_on_synthetic(species, tagset, chain, orientation, L, sub, nrate, junk):
     info = tags.load(species, tagset, chain)
     n = 200000
