@@ -1121,12 +1121,11 @@ struct dcb_ctx {
     char* stage[2] = {nullptr, nullptr};
     size_t stage_cap[2] = {0, 0};
     cudaEvent_t ev_stage[2] = {nullptr, nullptr};
-    // the host's share of dcb_decombine_ascii: chunks of clean reads packed by the host threads (dcb_pack_words) into
-    // page-locked buffers while the copy engine is busy with the text of a chunk the device packs
+    // pageable text in dcb_decombine_ascii: chunks of clean reads packed by the host threads (dcb_pack_words) into
+    // page-locked buffers, two so that the threads fill one while the copy engine takes the other
     uint32_t* hwords[2] = {nullptr, nullptr};
     size_t hwords_cap[2] = {0, 0};
-    cudaEvent_t ev_hw[2] = {nullptr, nullptr}, ev_acopy = nullptr;
-    bool acopy_pending = false;
+    cudaEvent_t ev_hw[2] = {nullptr, nullptr};
     uint32_t host_chunks = 0, device_chunks = 0;   // of the last dcb_decombine_ascii call
     // two-ended sharing (ascii_two_ended): the device takes the chunks from the front, a host thread packs chunks from the
     // back into ONE page-locked region (slot i = the i-th chunk from the end) until the two meet
@@ -1337,7 +1336,6 @@ dcb_ctx* dcb_ctx_create(int device, const dcb_tagset* v, const dcb_tagset* j, co
         if (cudaEventCreateWithFlags(&c->ev_scan[i], cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&c->ev_stage[i], cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&c->ev_hw[i], cudaEventDisableTiming) != cudaSuccess) return fail("cudaEventCreate");
-    if (cudaEventCreateWithFlags(&c->ev_acopy, cudaEventDisableTiming) != cudaSuccess) return fail("cudaEventCreate");
     for (int i = 0; i < 2; i++)
         if (cudaEventCreateWithFlags(&c->ev_text[i], cudaEventDisableTiming) != cudaSuccess) return fail("cudaEventCreate");
     return c;
@@ -1364,7 +1362,6 @@ void dcb_ctx_destroy(dcb_ctx* c) {
         if (c->ev_hw[i]) cudaEventDestroy(c->ev_hw[i]);
         if (c->hwords[i]) cudaFreeHost(c->hwords[i]);
     }
-    if (c->ev_acopy) cudaEventDestroy(c->ev_acopy);
     for (int i = 0; i < 2; i++) if (c->ev_text[i]) cudaEventDestroy(c->ev_text[i]);
     if (c->hstage) cudaFreeHost(c->hstage);
     if (c->stream3) { cudaStreamSynchronize(c->stream3); cudaStreamDestroy(c->stream3); }
@@ -1590,6 +1587,37 @@ static int read_counters(dcb_ctx* c, cudaStream_t s, uint64_t* counters) {
     return DCB_OK;
 }
 
+// Reads per chunk of the chunked paths: at least base, few enough chunks for the kMaxChunks queue counters, a multiple of 1024.
+static uint32_t chunk_reads(uint32_t base, uint64_t n) {
+    const uint32_t chunk = std::max<uint32_t>(base, (uint32_t)((n + kMaxChunks - 1) / kMaxChunks));
+    return (chunk + 1023u) & ~1023u;
+}
+
+// The chunk's kernels (chunk_no: its queue counters) and, when out is given, its result records back to the host.
+static int run_chunk(dcb_ctx* c, cudaStream_t s, uint32_t first, uint32_t count, int chunk_no, dcb_result* out) {
+    int rc;
+    if ((rc = launch_range(c, s, first, count, chunk_no, false))) return rc;
+    if (out)
+        CUDA_TRY(cudaMemcpyAsync(out + first, (dcb_result*)c->results.p + first, (size_t)count * sizeof(dcb_result),
+                                 cudaMemcpyDeviceToHost, s));
+    return DCB_OK;
+}
+
+// The chunked paths alternate the chunks between st[0] and st[1]: st[1] starts behind what st[0] has queued so far, and
+// st[0] ends behind all of st[1].  ran: the kernels ran; the context says so and the counters are added (synchronous).
+static int fork_streams(dcb_ctx* c, const cudaStream_t st[2]) {
+    CUDA_TRY(cudaEventRecord(c->ev_ready, st[0]));
+    CUDA_TRY(cudaStreamWaitEvent(st[1], c->ev_ready, 0));
+    return DCB_OK;
+}
+static int join_streams(dcb_ctx* c, const cudaStream_t st[2], bool ran, uint64_t* counters) {
+    CUDA_TRY(cudaEventRecord(c->ev_done, st[1]));
+    CUDA_TRY(cudaStreamWaitEvent(st[0], c->ev_done, 0));
+    if (!ran) return DCB_OK;
+    c->ran = true;
+    return read_counters(c, st[0], counters);
+}
+
 int dcb_upload(dcb_ctx* c, const dcb_packed* P) {
     if (!c || !P) { dcb_set_error("dcb_upload: null argument"); return DCB_EINVAL; }
     CUDA_TRY(cudaSetDevice(c->device));
@@ -1635,25 +1663,17 @@ int dcb_decombine_batch(dcb_ctx* c, const dcb_packed* P, dcb_result* out, uint64
     cudaStream_t st[2] = {c->stream, c->stream2};
     CUDA_TRY(cudaMemsetAsync(c->d_queue_count, 0, kZeroBlockBytes, st[0]));
     if ((rc = copy_side_arrays(c, P, st[0]))) return rc;
-    CUDA_TRY(cudaEventRecord(c->ev_ready, st[0]));
-    CUDA_TRY(cudaStreamWaitEvent(st[1], c->ev_ready, 0));
-    uint32_t chunk = std::max<uint32_t>(kChunkReads, (n + kMaxChunks - 1) / kMaxChunks);
-    chunk = (chunk + 1023u) & ~1023u;
+    if ((rc = fork_streams(c, st))) return rc;
+    const uint32_t chunk = chunk_reads(kChunkReads, n);
     int k = 0;
     for (uint32_t first = 0; first < n; first += chunk, k++) {
         const uint32_t count = std::min<uint32_t>(chunk, n - first);
         cudaStream_t s = st[k & 1];
         CUDA_TRY(cudaMemcpyAsync((uint32_t*)c->words.p + (size_t)first * sw, P->words + (size_t)first * sw, (size_t)count * sw * 4,
                                  cudaMemcpyHostToDevice, s));
-        if ((rc = launch_range(c, s, first, count, k, false))) return rc;
-        if (out)
-            CUDA_TRY(cudaMemcpyAsync(out + first, (dcb_result*)c->results.p + first, (size_t)count * sizeof(dcb_result),
-                                     cudaMemcpyDeviceToHost, s));
+        if ((rc = run_chunk(c, s, first, count, k, out))) return rc;
     }
-    CUDA_TRY(cudaEventRecord(c->ev_done, st[1]));
-    CUDA_TRY(cudaStreamWaitEvent(st[0], c->ev_done, 0));
-    c->ran = true;
-    return read_counters(c, st[0], counters);
+    return join_streams(c, st, true, counters);
 }
 
 // ---- ASCII in: pack on the device ----------------------------------------------------------------------------
@@ -1677,9 +1697,6 @@ static int ascii_geometry(const uint32_t* len, uint64_t n, uint32_t uniform_len,
     return DCB_OK;
 }
 
-// Pack reads [first, first + count) on stream s (buffers of parity `par`): text bytes and offsets / lengths up, the pack
-// kernel, the scan that continues the exception index from the chunks before (ordered across the two streams by
-// events), the exception entries.  The packed data lands in the context's batch buffers at the reads' global positions.
 // Host threads this process may use for packing / gathering: all of them, or its part when several ranks share the host
 // (torchrun sets LOCAL_WORLD_SIZE).
 static int local_world() {
@@ -1693,12 +1710,52 @@ static int host_threads() {
     return std::max(1, std::min(32, t));
 }
 
-static int submit_host_chunk(dcb_ctx* c, cudaStream_t s, const uint32_t* hw, bool with_lens, uint32_t first, uint32_t count, int chunk_no);
-static int copy_host_chunk(dcb_ctx* c, cudaStream_t s, const uint32_t* hw, bool with_lens, uint32_t first, uint32_t count);
-// The host's share: the chunk's reads packed by the host threads into a page-locked buffer and copied to their slots --
-// a quarter of the text's bytes over the link.  Only for chunks of nothing but A / C / G / T (no exception list to merge:
-// the chunk's groups take part in the running exception index with a count of zero).  1: done, 0: not clean (the caller
-// lets the device pack the chunk), < 0: error.
+// The scan that continues the exception index over the chunk's groups from where chunk chunk_no - 1 ends (ordered
+// across the two streams by events).
+static int scan_chunk(dcb_ctx* c, cudaStream_t s, uint32_t first, uint32_t groups, int chunk_no) {
+    if (chunk_no > 0) CUDA_TRY(cudaStreamWaitEvent(s, c->ev_scan[(chunk_no - 1) & 1], 0));
+    dcb_pack_scan_kernel<<<1, 1024, 0, s>>>((const uint32_t*)c->group_count.p, first >> 5, groups, (uint32_t*)c->exc_index.p, c->d_exc_total);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaEventRecord(c->ev_scan[chunk_no & 1], s));
+    return DCB_OK;
+}
+
+// Reads [first, first + count) packed by the host threads (dcb_pack_words) into hw, page-locked: the words, then (reads
+// of varying length, len != NULL) the 16-bit lengths behind them.  1: packed, 0: not clean (a symbol beyond A / C / G / T,
+// or no AVX2: the device packs the chunk), < 0: error.
+static int pack_words_host(const char* ascii, const uint64_t* off, const uint32_t* len, uint32_t uniform_len, int revcomp,
+                           uint32_t sw, uint64_t first, uint32_t count, int threads, uint32_t* hw) {
+    int clean = 0;
+    const int rc = dcb_pack_words(ascii, off, len, first, count, uniform_len, revcomp, sw, hw, threads, &clean);
+    if (rc) return rc;
+    if (!clean) return 0;
+    if (len) {
+        uint16_t* hl = reinterpret_cast<uint16_t*>(reinterpret_cast<char*>(hw) + (size_t)count * sw * 4);
+        for (uint32_t i = 0; i < count; i++) hl[i] = (uint16_t)len[first + i];
+    }
+    return 1;
+}
+
+// A chunk pack_words_host packed, copied to its slots: a quarter of the text's bytes over the link.
+static int copy_host_chunk(dcb_ctx* c, cudaStream_t s, const uint32_t* hw, bool with_lens, uint32_t first, uint32_t count) {
+    const uint32_t sw = c->batch.slot_words;
+    const size_t wbytes = (size_t)count * sw * 4;
+    CUDA_TRY(cudaMemcpyAsync((uint32_t*)c->words.p + (size_t)first * sw, hw, wbytes, cudaMemcpyHostToDevice, s));
+    if (with_lens)
+        CUDA_TRY(cudaMemcpyAsync((uint16_t*)c->lens.p + first, reinterpret_cast<const char*>(hw) + wbytes, (size_t)count * 2, cudaMemcpyHostToDevice, s));
+    return DCB_OK;
+}
+
+// A host-packed chunk has no exception list to merge: its groups join the running exception index with a count of zero.
+static int index_host_chunk(dcb_ctx* c, cudaStream_t s, uint32_t first, uint32_t count, int chunk_no) {
+    const uint32_t groups = (count + 31) / 32;
+    CUDA_TRY(cudaMemsetAsync((uint32_t*)c->flags.p + (first >> 5), 0, (size_t)groups * 4, s));
+    CUDA_TRY(cudaMemsetAsync((uint32_t*)c->group_count.p + (first >> 5), 0, (size_t)groups * 4, s));
+    return scan_chunk(c, s, first, groups, chunk_no);
+}
+
+// The chunk packed by the host threads into the page-locked buffer of parity par, copied to its slots and indexed on
+// stream s.  1: done, 0: not clean (the caller lets the device pack the chunk), < 0: error.
 static int pack_chunk_host(dcb_ctx* c, cudaStream_t s, int par, const char* ascii, const uint64_t* off, const uint32_t* len,
                            uint32_t uniform_len, int revcomp, uint32_t first, uint32_t count, int chunk_no) {
     const uint32_t sw = c->batch.slot_words;
@@ -1711,42 +1768,17 @@ static int pack_chunk_host(dcb_ctx* c, cudaStream_t s, int par, const char* asci
         if (cudaHostAlloc((void**)&c->hwords[par], want, cudaHostAllocDefault) != cudaSuccess) { (void)cudaGetLastError(); return 0; }
         c->hwords_cap[par] = want;
     }
-    int clean = 0;
-    int rc = dcb_pack_words(ascii, off, len, first, count, uniform_len, revcomp, sw, c->hwords[par], host_threads(), &clean);
-    if (rc) return rc;
-    if (!clean) return 0;
-    if (len) {
-        uint16_t* hl = reinterpret_cast<uint16_t*>(reinterpret_cast<char*>(c->hwords[par]) + wbytes);
-        for (uint32_t i = 0; i < count; i++) hl[i] = (uint16_t)len[first + i];
-    }
-    if ((rc = submit_host_chunk(c, s, c->hwords[par], len != nullptr, first, count, chunk_no))) return rc;
+    int rc = pack_words_host(ascii, off, len, uniform_len, revcomp, sw, first, count, host_threads(), c->hwords[par]);
+    if (rc != 1) return rc;
+    if ((rc = copy_host_chunk(c, s, c->hwords[par], len != nullptr, first, count))) return rc;
+    if ((rc = index_host_chunk(c, s, first, count, chunk_no))) return rc;
     CUDA_TRY(cudaEventRecord(c->ev_hw[par], s));
     return 1;
 }
 
-// A chunk the host threads packed -- words, then (reads of varying length) the 16-bit lengths behind them, in page-locked
-// memory -- copied to its slots; its groups join the running exception index with a count of zero.
-static int copy_host_chunk(dcb_ctx* c, cudaStream_t s, const uint32_t* hw, bool with_lens, uint32_t first, uint32_t count) {
-    const uint32_t sw = c->batch.slot_words;
-    const size_t wbytes = (size_t)count * sw * 4;
-    CUDA_TRY(cudaMemcpyAsync((uint32_t*)c->words.p + (size_t)first * sw, hw, wbytes, cudaMemcpyHostToDevice, s));
-    if (with_lens)
-        CUDA_TRY(cudaMemcpyAsync((uint16_t*)c->lens.p + first, reinterpret_cast<const char*>(hw) + wbytes, (size_t)count * 2, cudaMemcpyHostToDevice, s));
-    return DCB_OK;
-}
-// hw == nullptr: the words (and lengths) are there already (copy_host_chunk on another stream, which s has been made to wait for)
-static int submit_host_chunk(dcb_ctx* c, cudaStream_t s, const uint32_t* hw, bool with_lens, uint32_t first, uint32_t count, int chunk_no) {
-    if (hw) { const int rc = copy_host_chunk(c, s, hw, with_lens, first, count); if (rc) return rc; }
-    const uint32_t groups = (count + 31) / 32;
-    CUDA_TRY(cudaMemsetAsync((uint32_t*)c->flags.p + (first >> 5), 0, (size_t)groups * 4, s));
-    CUDA_TRY(cudaMemsetAsync((uint32_t*)c->group_count.p + (first >> 5), 0, (size_t)groups * 4, s));
-    if (chunk_no > 0) CUDA_TRY(cudaStreamWaitEvent(s, c->ev_scan[(chunk_no - 1) & 1], 0));
-    dcb_pack_scan_kernel<<<1, 1024, 0, s>>>((const uint32_t*)c->group_count.p, first >> 5, groups, (uint32_t*)c->exc_index.p, c->d_exc_total);
-    CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaEventRecord(c->ev_scan[chunk_no & 1], s));
-    return DCB_OK;
-}
-
+// Pack reads [first, first + count) on stream s (buffers of parity `par`): text bytes and offsets / lengths up, the pack
+// kernel, the scan that continues the exception index, the exception entries.  The packed data lands in the context's
+// batch buffers at the reads' global positions.
 static int pack_chunk(dcb_ctx* c, cudaStream_t s, int par, const char* ascii, const uint64_t* off, const uint32_t* len,
                       uint32_t uniform_len, int revcomp, uint32_t first, uint32_t count, size_t exc_cap, int chunk_no,
                       bool staged = false) {
@@ -1808,8 +1840,6 @@ static int pack_chunk(dcb_ctx* c, cudaStream_t s, int par, const char* ascii, co
     } else {
         if ((rc = c->text[par].ensure(hi - lo + 64))) return rc;
         CUDA_TRY(cudaMemcpyAsync(c->text[par].p, ascii + lo, hi - lo, cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaEventRecord(c->ev_acopy, s));
-        c->acopy_pending = true;
         CUDA_TRY(cudaEventRecord(c->ev_text[par], s));
         c->text_pending[par] = true;
         src.text = (const unsigned char*)c->text[par].p; src.text_lo = lo;
@@ -1829,10 +1859,7 @@ static int pack_chunk(dcb_ctx* c, cudaStream_t s, int par, const char* ascii, co
     dcb_pack_kernel<<<blocks, 256, 0, s>>>(src, revcomp, sw, (uint32_t*)c->words.p, (uint16_t*)c->lens.p, (uint32_t*)c->flags.p,
                                            (uint32_t*)c->group_count.p);
     CUDA_TRY(cudaGetLastError());
-    if (chunk_no > 0) CUDA_TRY(cudaStreamWaitEvent(s, c->ev_scan[(chunk_no - 1) & 1], 0));   // the list continues where the chunk before ends
-    dcb_pack_scan_kernel<<<1, 1024, 0, s>>>((const uint32_t*)c->group_count.p, first >> 5, groups, (uint32_t*)c->exc_index.p, c->d_exc_total);
-    CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaEventRecord(c->ev_scan[chunk_no & 1], s));
+    if ((rc = scan_chunk(c, s, first, groups, chunk_no))) return rc;
     dcb_pack_exc_kernel<<<blocks, 256, 0, s>>>(src, revcomp, sw, (const uint32_t*)c->flags.p, (const uint32_t*)c->exc_index.p, (uint32_t)exc_cap,
                                                (uint32_t*)c->exc_read.p, (uint16_t*)c->exc_pos.p, (uint8_t*)c->exc_kind.p);
     CUDA_TRY(cudaGetLastError());
@@ -1922,17 +1949,12 @@ static int ascii_two_ended(dcb_ctx* c, const char* ascii, const uint64_t* off, c
             }
             const uint32_t count = count_of(k);
             uint32_t* hw = slot_of(k);
-            int clean = 0;
-            const int rc = dcb_pack_words(ascii, off, lens, first_of(k), count, uniform_len, revcomp, sw, hw, nt, &clean);
-            if (rc || !clean) {
+            const int rc = pack_words_host(ascii, off, lens, uniform_len, revcomp, sw, first_of(k), count, nt, hw);
+            if (rc != 1) {
                 std::lock_guard<std::mutex> g(m);
-                if (rc) worker_rc = rc;
+                if (rc < 0) worker_rc = rc;
                 dirty[k] = 1; host_open = false;
                 return;
-            }
-            if (lens) {
-                uint16_t* hl = reinterpret_cast<uint16_t*>(reinterpret_cast<char*>(hw) + (size_t)count * sw * 4);
-                for (uint32_t i = 0; i < count; i++) hl[i] = (uint16_t)lens[first_of(k) + i];
             }
             // the packed words go to their slots right away, between the device's text copies: only the chunk's place in
             // the exception index and its kernels have to wait for the chunks in front of it
@@ -1957,9 +1979,7 @@ static int ascii_two_ended(dcb_ctx* c, const char* ascii, const uint64_t* off, c
         int r;
         if ((r = pack_chunk(c, s, k & 1, ascii, off, lens, uniform_len, revcomp, first, count, exc_cap, k, false))) return r;
         c->device_chunks++;
-        if ((r = launch_range(c, s, first, count, k, false))) return r;
-        if (out) CUDA_TRY(cudaMemcpyAsync(out + first, (dcb_result*)c->results.p + first, (size_t)count * sizeof(dcb_result), cudaMemcpyDeviceToHost, s));
-        return DCB_OK;
+        return run_chunk(c, s, first, count, k, out);
     };
     c->text_pending[0] = c->text_pending[1] = false;
     int k = 0;
@@ -1987,24 +2007,35 @@ static int ascii_two_ended(dcb_ctx* c, const char* ascii, const uint64_t* off, c
         cudaStream_t s = st[k & 1];
         const uint32_t first = (uint32_t)first_of(k), count = count_of(k);
         CUDA_TRY(cudaStreamWaitEvent(s, c->ev_hcopy[k], 0));
-        if ((rc = submit_host_chunk(c, s, nullptr, lens != nullptr, first, count, k))) return rc;
+        if ((rc = index_host_chunk(c, s, first, count, k))) return rc;
         c->host_chunks++;
-        if ((rc = launch_range(c, s, first, count, k, false))) return rc;
-        if (out) CUDA_TRY(cudaMemcpyAsync(out + first, (dcb_result*)c->results.p + first, (size_t)count * sizeof(dcb_result), cudaMemcpyDeviceToHost, s));
+        if ((rc = run_chunk(c, s, first, count, k, out))) return rc;
     }
     return DCB_OK;
 }
 
 int dcb_decombine_ascii(dcb_ctx* c, const char* ascii, const uint64_t* off, const uint32_t* len, uint64_t n, uint32_t uniform_len,
                         int revcomp, dcb_result* out, uint64_t* counters) {
+    // Who packs a chunk: the device (the text goes over the link, 4 bytes per packed byte) or the host threads.  Text in
+    // pageable memory would have to be gathered into page-locked staging by the host threads anyway: they pack it instead,
+    // until a chunk holds a symbol beyond A / C / G / T.  Page-locked text: shared from both ends (ascii_two_ended) -- also
+    // with several ranks on one host, each with its share of the host threads (LOCAL_WORLD_SIZE): measured on 2 ranks
+    // 407 -> 528 M reads/s, on 8 ranks 655 -> 686 M (there the host's memory system bounds the copies of all eight links
+    // and the packer takes 11 of 39 chunks).  DCB_HOST_SHARE=0: the device packs every chunk (measurements, tests).
+    const char* hs = std::getenv("DCB_HOST_SHARE");
+    if (hs && std::strcmp(hs, "0") && std::strcmp(hs, "1")) {
+        dcb_set_error("DCB_HOST_SHARE=%s: accepted values are 1 (the default: chunks shared between the host threads and the "
+                      "device) and 0 (the device packs every chunk)", hs);
+        return DCB_EINVAL;
+    }
+    const bool host_share = !hs || hs[0] == '1';
     size_t exc_cap = 0;
     int rc;
     if ((rc = ascii_begin(c, ascii, off, len, n, uniform_len, &exc_cap))) return rc;
     const uint32_t* lens = uniform_len ? nullptr : len;
     cudaStream_t st[2] = {c->stream, c->stream2};
     CUDA_TRY(cudaMemsetAsync(c->d_queue_count, 0, kZeroBlockBytes, st[0]));
-    CUDA_TRY(cudaEventRecord(c->ev_ready, st[0]));
-    CUDA_TRY(cudaStreamWaitEvent(st[1], c->ev_ready, 0));
+    if ((rc = fork_streams(c, st))) return rc;
     // text in pageable memory (a memory-mapped file): smaller chunks through page-locked staging buffers
     bool staged = false;
     if (n) {
@@ -2012,27 +2043,13 @@ int dcb_decombine_ascii(dcb_ctx* c, const char* ascii, const uint64_t* off, cons
         if (cudaPointerGetAttributes(&attr, ascii) != cudaSuccess) { (void)cudaGetLastError(); staged = true; }
         else staged = attr.type == cudaMemoryTypeUnregistered;
     }
-    uint32_t chunk = std::max<uint32_t>(staged ? kChunkReads / 2 : kChunkReads, (uint32_t)((n + kMaxChunks - 1) / kMaxChunks));
-    chunk = (chunk + 1023u) & ~1023u;
-    // Who packs a chunk: the device (the text goes over the link, 4 bytes per packed byte) or the host threads.  Text in
-    // pageable memory would have to be gathered into page-locked staging by the host threads anyway: they pack it instead.
-    // Page-locked text: shared from both ends (ascii_two_ended) -- also with several ranks on one host, each with its share
-    // of the host threads (LOCAL_WORLD_SIZE): measured on 2 ranks 407 -> 528 M reads/s, on 8 ranks 655 -> 686 M (there the
-    // host's memory system bounds the copies of all eight links and the packer takes 11 of 39 chunks).
-    // DCB_HOST_SHARE=0 / 1 / 2 / 3: never / when the copy engine is busy / always / pageable text only (tests, measurements).
-    int host_share = 1;
-    if (const char* e = std::getenv("DCB_HOST_SHARE")) host_share = std::atoi(e);
     c->host_chunks = c->device_chunks = 0;
-    c->acopy_pending = false;
-    bool host_ok = host_share != 0, shared = false;
-    int k = 0;
-    const char* two = std::getenv("DCB_TWO_ENDED");          // 0: the round's earlier scheme (the caller's thread packs; measurements)
-    if (host_share == 1 && !staged && n && !(two && two[0] == '0')) {
+    bool shared = false;
+    if (host_share && !staged && n) {
         // smaller chunks: the shares are settled chunk by chunk, and the two sides meet inside one
         uint32_t fine = kChunkReads / 4;
         if (const char* e = std::getenv("DCB_CHUNK_READS")) fine = (uint32_t)std::max(1024, std::atoi(e));
-        fine = std::max<uint32_t>(fine, (uint32_t)((n + kMaxChunks - 1) / kMaxChunks));
-        fine = (fine + 1023u) & ~1023u;
+        fine = chunk_reads(fine, n);
         if ((n + fine - 1) / fine >= 4) {
             if ((rc = ascii_two_ended(c, ascii, off, lens, n, uniform_len, revcomp, out, fine, exc_cap))) {
                 cudaStreamSynchronize(st[0]); cudaStreamSynchronize(st[1]);
@@ -2042,38 +2059,24 @@ int dcb_decombine_ascii(dcb_ctx* c, const char* ascii, const uint64_t* off, cons
             shared = true;
         }
     }
+    const uint32_t chunk = chunk_reads(staged ? kChunkReads / 2 : kChunkReads, n);
+    bool host_ok = host_share && staged;
+    int k = 0;
     for (uint64_t first = 0; first < n && !shared; first += chunk, k++) {
         const uint32_t count = (uint32_t)std::min<uint64_t>(chunk, n - first);
         cudaStream_t s = st[k & 1];
-        bool by_host = false;
         if (host_ok) {
-            bool want = staged || host_share == 2;
-            if (!want && host_share == 1 && c->acopy_pending) {
-                const cudaError_t q = cudaEventQuery(c->ev_acopy);
-                if (q == cudaErrorNotReady) want = true;
-                else if (q != cudaSuccess) { dcb_set_error("cudaEventQuery failed: %s", cudaGetErrorString(q)); return DCB_ENOGPU; }
-            }
-            if (want) {
-                rc = pack_chunk_host(c, s, k & 1, ascii, off, lens, uniform_len, revcomp, (uint32_t)first, count, k);
-                if (rc < 0) return rc;
-                by_host = rc == 1;
-                if (!by_host) host_ok = false;          // symbols beyond A / C / G / T (or no AVX2): the device packs the rest
-            }
+            if ((rc = pack_chunk_host(c, s, k & 1, ascii, off, lens, uniform_len, revcomp, (uint32_t)first, count, k)) < 0) return rc;
+            host_ok = rc == 1;                          // not clean: the device packs this chunk and the rest
         }
-        if (by_host) c->host_chunks++;
+        if (host_ok) c->host_chunks++;
         else {
             if ((rc = pack_chunk(c, s, k & 1, ascii, off, lens, uniform_len, revcomp, (uint32_t)first, count, exc_cap, k, staged))) return rc;
             c->device_chunks++;
         }
-        if ((rc = launch_range(c, s, (uint32_t)first, count, k, false))) return rc;
-        if (out)
-            CUDA_TRY(cudaMemcpyAsync(out + first, (dcb_result*)c->results.p + first, (size_t)count * sizeof(dcb_result),
-                                     cudaMemcpyDeviceToHost, s));
+        if ((rc = run_chunk(c, s, (uint32_t)first, count, k, out))) return rc;
     }
-    CUDA_TRY(cudaEventRecord(c->ev_done, st[1]));
-    CUDA_TRY(cudaStreamWaitEvent(st[0], c->ev_done, 0));
-    c->ran = true;
-    if ((rc = read_counters(c, st[0], counters))) return rc;
+    if ((rc = join_streams(c, st, true, counters))) return rc;
     return ascii_finish(c, exc_cap, nullptr);
 }
 
@@ -2089,16 +2092,14 @@ int dcb_pack_device(dcb_ctx* c, const char* ascii, const uint64_t* off, const ui
     cudaStream_t st[2] = {c->stream, c->stream2};
     cudaEvent_t e0, e1;
     CUDA_TRY(cudaEventCreate(&e0)); CUDA_TRY(cudaEventCreate(&e1));
-    CUDA_TRY(cudaEventRecord(c->ev_ready, st[0]));
-    CUDA_TRY(cudaStreamWaitEvent(st[1], c->ev_ready, 0));
+    if ((rc = fork_streams(c, st))) return rc;
     const uint32_t chunk = kChunkReads;
     int k = 0;
     CUDA_TRY(cudaEventRecord(e0, st[0]));
     for (uint64_t first = 0; first < n; first += chunk, k++)
         if ((rc = pack_chunk(c, st[k & 1], k & 1, ascii, off, lens, uniform_len, revcomp, (uint32_t)first,
                              (uint32_t)std::min<uint64_t>(chunk, n - first), exc_cap, k))) return rc;
-    CUDA_TRY(cudaEventRecord(c->ev_done, st[1]));
-    CUDA_TRY(cudaStreamWaitEvent(st[0], c->ev_done, 0));
+    if ((rc = join_streams(c, st, false, nullptr))) return rc;
     CUDA_TRY(cudaEventRecord(e1, st[0]));
     CUDA_TRY(cudaStreamSynchronize(st[0]));
     float ms = 0.f;

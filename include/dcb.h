@@ -254,7 +254,10 @@ int dcb_decombine_batch(dcb_ctx*, const dcb_packed* reads, dcb_result* out, uint
  * the host.  Read i is ascii[off[i] .. off[i] + len[i]); offsets must not decrease inside the batch (FASTQ order).
  * off == NULL: the reads are contiguous, read i at i * uniform_len.  uniform_len != 0: every read has that length and
  * len is ignored.  Chunks of nothing but A / C / G / T are shared between the device packer and the host threads
- * (dcb_pack_words), whichever is free; reads with other symbols are packed by the device. */
+ * (dcb_pack_words): page-locked text from both ends, the device taking chunks from the front and the host threads from
+ * the back; pageable text by the host threads until the first chunk with another symbol.  Chunks with other symbols are
+ * packed by the device.  The environment variable DCB_HOST_SHARE = 0 makes the device pack every chunk; a value other
+ * than 0 or 1 fails the call with DCB_EINVAL. */
 int dcb_decombine_ascii(dcb_ctx*, const char* ascii, const uint64_t* off, const uint32_t* len, uint64_t n, uint32_t uniform_len,
                         int revcomp, dcb_result* out, uint64_t* counters);
 /* The device packer alone: its output copied back into a host dcb_packed (free with dcb_packed_free); tests compare it
@@ -263,8 +266,8 @@ int dcb_pack_device(dcb_ctx*, const char* ascii, const uint64_t* off, const uint
                     int revcomp, dcb_packed** out);
 int dcb_pack_device_ms(dcb_ctx*, double* ms);
 /* How the chunks of the last dcb_decombine_ascii call were packed: by the host threads (clean reads, dcb_pack_words: a
- * quarter of the text's bytes cross the link) or by the device (the text itself crosses the link).  The environment
- * variable DCB_HOST_SHARE = 0 / 2 forces never / always (default: the host packs while the copy engine is busy). */
+ * quarter of the text's bytes cross the link) or by the device (the text itself crosses the link).  With
+ * DCB_HOST_SHARE = 0 the host packs none. */
 int dcb_last_pack_shares(dcb_ctx*, uint32_t* host_chunks, uint32_t* device_chunks);
 
 /* Page-locked host memory for result records (so that the device->host copies of dcb_decombine_batch run

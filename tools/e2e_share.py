@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""e2e of dcb_decombine_ascii (ASCII reads in page-locked host memory -> records in host memory) under the chunk-sharing
-variants: DCB_TWO_ENDED=0 (the caller's thread packs every other chunk) against the two-ended scheme at several chunk sizes.
+"""e2e of dcb_decombine_ascii (ASCII reads in page-locked host memory -> records in host memory) with the chunks shared
+from both ends at several chunk sizes, against the device packing every chunk.
 usage (GPU box): python tools/e2e_share.py [reads]"""
 import json
 import os
@@ -21,11 +21,10 @@ r1, _ = syn.reads(0, n)
 text = _lib.PinnedBytes(r1)
 ctx = _lib.Context(vt, jt, device=0)
 want = None
-for name, env in (("caller packs every other chunk", {"DCB_TWO_ENDED": "0"}),
-                  ("two-ended, 128 K", {"DCB_CHUNK_READS": "131072"}), ("two-ended, 256 K", {"DCB_CHUNK_READS": "262144"}),
+for name, env in (("two-ended, 128 K", {"DCB_CHUNK_READS": "131072"}), ("two-ended, 256 K", {"DCB_CHUNK_READS": "262144"}),
                   ("two-ended, 512 K", {"DCB_CHUNK_READS": "524288"}), ("two-ended, 1 M", {"DCB_CHUNK_READS": "1048576"}),
-                  ("device only", {"DCB_HOST_SHARE": "0"}), ("host only", {"DCB_HOST_SHARE": "2"})):
-    for k in ("DCB_TWO_ENDED", "DCB_CHUNK_READS", "DCB_HOST_SHARE"):
+                  ("device only", {"DCB_HOST_SHARE": "0"})):
+    for k in ("DCB_CHUNK_READS", "DCB_HOST_SHARE"):
         os.environ.pop(k, None)
     os.environ.update(env)
     for _ in range(3):
