@@ -1139,6 +1139,7 @@ struct dcb_ctx {
     int vgen_words = 0, jgen_words = 0, vcore_words = 0, jcore_words = 0, vidx_words = 0, jidx_words = 0, uidx_words = 0;
     DevBuf words, lens, flags, exc_read, exc_pos, exc_kind, exc_index, results, queue;
     std::vector<uint32_t> h_exc_index;   // host copy of exc_index while its upload is in flight
+    uint32_t exc_cap = 0;                // entries of the device-side exception list of the batch being packed on the device
     uint32_t* d_queue_count = nullptr;
     unsigned long long* d_counters = nullptr;
     BatchDev batch{};
@@ -1711,10 +1712,12 @@ static int host_threads() {
 }
 
 // The scan that continues the exception index over the chunk's groups from where chunk chunk_no - 1 ends (ordered
-// across the two streams by events).
+// across the two streams by events).  Groups whose entries do not fit in the list lose their flag words (see
+// dcb_pack_scan_kernel): the kernels of the chunk, which run before ascii_finish fails the call, read no entry past it.
 static int scan_chunk(dcb_ctx* c, cudaStream_t s, uint32_t first, uint32_t groups, int chunk_no) {
     if (chunk_no > 0) CUDA_TRY(cudaStreamWaitEvent(s, c->ev_scan[(chunk_no - 1) & 1], 0));
-    dcb_pack_scan_kernel<<<1, 1024, 0, s>>>((const uint32_t*)c->group_count.p, first >> 5, groups, (uint32_t*)c->exc_index.p, c->d_exc_total);
+    dcb_pack_scan_kernel<<<1, 1024, 0, s>>>((const uint32_t*)c->group_count.p, first >> 5, groups, c->exc_cap, (uint32_t*)c->exc_index.p,
+                                            (uint32_t*)c->flags.p, c->d_exc_total);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaEventRecord(c->ev_scan[chunk_no & 1], s));
     return DCB_OK;
@@ -1877,6 +1880,7 @@ static int ascii_begin(dcb_ctx* c, const char* ascii, const uint64_t* off, const
     int rc;
     if ((rc = ascii_geometry(uniform_len ? nullptr : len, n, uniform_len, &G))) return rc;
     *exc_cap = exc_capacity(n);
+    c->exc_cap = (uint32_t)*exc_cap;
     if ((rc = prepare_batch(c, &G, *exc_cap))) return rc;
     if ((rc = c->group_count.ensure(((n + 31) / 32 + 2) * 4))) return rc;
     CUDA_TRY(cudaMemsetAsync(c->d_exc_total, 0, 16, c->stream));

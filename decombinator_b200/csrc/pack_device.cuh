@@ -118,9 +118,12 @@ dcb_pack_kernel(PackSrc src, int revcomp, uint32_t slot_words, uint32_t* __restr
 
 // exclusive scan of the chunk's group counts into the exception index, continuing from *carry (the entries written by
 // the chunks before); one block.  index[first_group + n_groups] = the new total, which is also left in *carry.
+// The list holds cap entries: the index values are clamped to cap, and a group whose run does not end inside the list
+// loses its flag word, so that pass 2 writes none of its entries and no decombine kernel looks for them.  *carry keeps the
+// true total (the host compares it with cap and fails the call).
 __global__ void __launch_bounds__(1024)
-dcb_pack_scan_kernel(const uint32_t* __restrict__ group_count, uint32_t first_group, uint32_t n_groups, uint32_t* __restrict__ index,
-                     uint32_t* __restrict__ carry) {
+dcb_pack_scan_kernel(const uint32_t* __restrict__ group_count, uint32_t first_group, uint32_t n_groups, uint32_t cap,
+                     uint32_t* __restrict__ index, uint32_t* __restrict__ flags, uint32_t* __restrict__ carry) {
     __shared__ uint32_t warp_sum[32];
     __shared__ uint32_t running;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -148,12 +151,16 @@ dcb_pack_scan_kernel(const uint32_t* __restrict__ group_count, uint32_t first_gr
         }
         __syncthreads();
         const uint32_t before = running + (wid ? warp_sum[wid - 1] : 0u) + incl - v;
-        if (k < n_groups) index[first_group + k] = before;
+        if (k < n_groups) {
+            const uint32_t at = min(before, cap);
+            index[first_group + k] = at;
+            if (v > cap - at) flags[first_group + k] = 0u;        // the run crosses or lies beyond the end of the list
+        }
         __syncthreads();
         if (tid == 1023) running = before + v;
         __syncthreads();
     }
-    if (tid == 0) { index[first_group + n_groups] = running; *carry = running; }
+    if (tid == 0) { index[first_group + n_groups] = min(running, cap); *carry = running; }
 }
 
 // pass 2: the entries of the flagged reads, in (read, position) order, at index[group] onwards
