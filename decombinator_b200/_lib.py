@@ -50,7 +50,9 @@ class CBcParams(ctypes.Structure):
 
 
 BC_OK, BC_FAIL_N, BC_FAIL_NOSPACER, BC_FAIL_NOT2, BC_FAIL_N1SHORT, BC_FAIL_N1LONG, BC_FAIL_N2END, BC_FAIL_QUALITY, BC_HOST = 0, 1, 2, 3, 4, 5, 6, 7, 255
-OLIGOS_ON_DEVICE = {"m13": 0, "i8": 1}
+OLIGOS_ON_DEVICE = {"m13": 0, "i8": 1, "i8_single": 2, "nebio": 3, "takara": 4}   # -ol (lower case) -> DCB_OLIGO_*
+BC_LENGTH = {"m13": 12, "i8": 12, "i8_single": 12, "nebio": 17, "takara": 12}      # symbols of the barcode dcb_barcodes assembles
+BC_FIXED = ("nebio", "takara")                  # designs whose barcode is a fixed slice of the region (no N1 / N2)
 
 
 class CSynthParams(ctypes.Structure):

@@ -372,14 +372,21 @@ def _device_barcodes(rows, inputargs, qp):
         return None      # (without the allowNs key the reference fails on the first barcode that holds an N: host path)
     status, n1, code = _gpu().barcodes([r[8] for r in rows], [r[9] for r in rows], _lib.OLIGOS_ON_DEVICE[name],
                                        inputargs["allowNs"] != False, qp[0], qp[1], qp[2])  # noqa: E712
-    sym = (code[:, None] >> (np.uint64(3) * np.arange(12, dtype=np.uint64))[None, :]) & np.uint64(7)
-    text = _BC_SYMBOLS[sym.astype(np.intp)].tobytes().decode("ascii")          # 12 characters per row, back to back
-    _count_device_barcodes(status, n1)
+    text = _decode_barcodes(code, _lib.BC_LENGTH[name])      # BC_LENGTH[name] characters per row, back to back
+    _count_device_barcodes(status, n1, name)
     return status, text
 
 
-def _count_device_barcodes(status, n1):
-    """The reference's counters for the rows decided on the device (collapse.py:241-278, 388-422, 546-553)."""
+def _decode_barcodes(code, width):
+    """dcb_barcodes codes of `width` symbols -> their barcode strings, back to back in one str."""
+    sym = (code[:, None] >> (np.uint64(3) * np.arange(width, dtype=np.uint64))[None, :]) & np.uint64(7)
+    return _BC_SYMBOLS[sym.astype(np.intp)].tobytes().decode("ascii")
+
+
+def _count_device_barcodes(status, n1, name):
+    """The reference's counters for the rows decided on the device (collapse.py:241-278, 388-422, 546-553).  The
+    fixed-barcode designs (NEBIO, TAKARA) have no N1: every placed row counts as getbarcode_pass_other, none as a short
+    or long barcode."""
     st = np.bincount(status, minlength=256)
     for key, k in (("getbarcode_fail_N", st[_lib.BC_FAIL_N]), ("getbarcode_fail_nospacerfound", st[_lib.BC_FAIL_NOSPACER]),
                    ("getbarcode_fail_not2spacersfound", st[_lib.BC_FAIL_NOT2]), ("getbarcode_fail_n1tooshort", st[_lib.BC_FAIL_N1SHORT]),
@@ -388,9 +395,13 @@ def _count_device_barcodes(status, n1):
                    ("readdata_fail_low_barcode_quality", st[_lib.BC_FAIL_QUALITY])):
         if k:
             counts[key] += int(k)
-    placed = (status == _lib.BC_OK) | (status == _lib.BC_FAIL_QUALITY)         # both spacers found exactly, N1 / N2 in range
-    for key, k in (("getbarcode_pass_exactmatch", placed.sum()), ("getbarcode_pass_other", (placed & (n1 == 6)).sum()),
-                   ("readdata_short_barcode", (placed & (n1 < 6)).sum()), ("readdata_long_barcode", (placed & (n1 > 6)).sum())):
+    placed = (status == _lib.BC_OK) | (status == _lib.BC_FAIL_QUALITY)         # spacers found exactly, N1 / N2 in range
+    if name in _lib.BC_FIXED:
+        other, short, long_ = placed, np.zeros_like(placed), np.zeros_like(placed)
+    else:
+        other, short, long_ = placed & (n1 == 6), placed & (n1 < 6), placed & (n1 > 6)
+    for key, k in (("getbarcode_pass_exactmatch", placed.sum()), ("getbarcode_pass_other", other.sum()),
+                   ("readdata_short_barcode", short.sum()), ("readdata_long_barcode", long_.sum())):
         if k:
             counts[key] += int(k)
 
@@ -451,14 +462,14 @@ def _filter_columns(data, inputargs, barcode_quality_parameters, first_index=0):
         return None
     status, n1, code = _gpu().barcodes_arrays(*data.barcode_columns(), _lib.OLIGOS_ON_DEVICE[name], inputargs["allowNs"] != False,  # noqa: E712
                                               *barcode_quality_parameters)
-    _count_device_barcodes(status, n1)
+    _count_device_barcodes(status, n1, name)
     ok, host = status == _lib.BC_OK, status == _lib.BC_HOST
     # rows whose barcode the kernel assembled: no Python row at all, the three strings collapse files them under come from
     # dcb_format_collapse_rows; rows it hands back (fuzzy spacer search) become Python rows as before
     seqs, dcrs, etcs = data.collapse_lines(ok)
-    sym = (code[ok][:, None] >> (np.uint64(3) * np.arange(12, dtype=np.uint64))[None, :]) & np.uint64(7)
-    text = _BC_SYMBOLS[sym.astype(np.intp)].tobytes().decode("ascii")
-    fast = (seqs, dcrs, etcs, re.findall("." * 12, text), (first_index + np.nonzero(ok)[0]).tolist())
+    width = _lib.BC_LENGTH[name]
+    text = _decode_barcodes(code[ok], width)
+    fast = (seqs, dcrs, etcs, re.findall("." * width, text), (first_index + np.nonzero(ok)[0]).tolist())
     rows = data.subset_rows(host) if bool(host.any()) else []
     return rows, (first_index + np.nonzero(host)[0]).tolist(), fast, int(len(status))
 
@@ -490,12 +501,13 @@ def _filter_rows(data, inputargs, barcode_quality_parameters, dont_count, from_f
     lenthreshold, sampling = inputargs["lenthreshold"], inputargs["sampling_analysis"]
     n_long = n_ok = 0
     HOST, OK = _lib.BC_HOST, _lib.BC_OK
+    width = _lib.BC_LENGTH.get(inputargs["oligo"].lower(), 0)
     for lcount, line in enumerate(rows):
         if lcount % 50000 == 0 and lcount != 0 and not dont_count:
             print("   Read in", lcount, "lines... ", round(time.time() - t0, 2), "seconds")
         st = status[lcount] if status is not None else HOST
         if st == OK:
-            barcode, barcode_qualstring = text[12 * lcount:12 * lcount + 12], None
+            barcode, barcode_qualstring = text[width * lcount:width * (lcount + 1)], None
         elif st != HOST:
             continue                                  # rejected on the device, counted in _device_barcodes
         else:
@@ -549,8 +561,9 @@ def _group_rows(kept, lev_threshold_fraction):
     the SAME barcode interact, so any partition of the barcodes (parallel.py: hash(barcode) % world) can be grouped
     independently and merged by ``tick`` afterwards.
 
-    The rules run in the library over columns (dcb_group, csrc/group.cpp) when every barcode is twelve symbols of ACGTNSL
-    and the sequences are plain ASCII -- the usual case; anything else through the same rules in Python (_BarcodeMachine).
+    The rules run in the library over columns (dcb_group, csrc/group.cpp) when the barcodes are all of one length (up to
+    UMI_MAX_LEN symbols of ACGTNSL) and the sequences are plain ASCII -- the usual case; anything else through the same
+    rules in Python (_BarcodeMachine).
     Either way each round resolves, in ONE GPU batch, every sequence verdict some barcode waits for."""
     native = _group_rows_native(kept, lev_threshold_fraction) if len(kept) >= 64 and os.environ.get("DCB_GROUP_NATIVE", "1") != "0" else None
     if native is not None:
@@ -589,12 +602,14 @@ def _group_rows_native(kept, lev_threshold_fraction):
         seqs = "\n".join(seq_l).encode("ascii")
     except UnicodeEncodeError:
         return None
-    if len(bcs) != 12 * n or seqs.count(b"\n") != n - 1:          # (a sequence that holds a newline: not the library's shape)
+    width = len(bc_l[0])                                              # 12, or 17 for NEBIO
+    # (a sequence that holds a newline: not the library's shape)
+    if not 0 < width <= _lib.UMI_MAX_LEN or len(bcs) != width * n or seqs.count(b"\n") != n - 1:
         return None
-    sym = _BC_CODE[np.frombuffer(bcs, dtype=np.uint8)].reshape(n, 12)
+    sym = _BC_CODE[np.frombuffer(bcs, dtype=np.uint8)].reshape(n, width)
     if int(sym.max()) > 6 or len(set(map(len, bc_l))) != 1:
         return None
-    code = (sym.astype(np.uint64) << (np.uint64(3) * np.arange(12, dtype=np.uint64))[None, :]).sum(axis=1, dtype=np.uint64)
+    code = (sym.astype(np.uint64) << (np.uint64(3) * np.arange(width, dtype=np.uint64))[None, :]).sum(axis=1, dtype=np.uint64)
     g = _lib.Grouping(seqs, code, np.fromiter(idx_l, dtype=np.uint64, count=n))
     try:
         g.run(lambda symbols, off, ln, a, b: _gpu().lev_leq(symbols, off, ln, a, b, lev_threshold_fraction))

@@ -289,16 +289,21 @@ dcb_lev_leq_kernel(const uint8_t* __restrict__ sym, const uint64_t* __restrict__
 
 // ---- barcode extraction (SURVEY 8(f) row 3) ------------------------------------------------------------------------
 // One thread per decombined row: the barcode region (R2[:bclength], field 8 of an .n12 row) and its quality string.
-// What collapse.py does per row before any grouping, for the two-spacer oligos (M13, I8):
-//   get_barcode_positions (collapse.py:367-479): an 'N' anywhere rejects the row (unless -N); spacer 1 is searched in
-//     bc[0 : 10 + len(spacer1)] and must be found exactly once, spacer 2 in bc[len(spacer1):] and must be found exactly once
-//     (regex.findall: leftmost, non-overlapping); N1 lies between the spacers, N2 is the six bases behind spacer 2; N1 of
-//     <= 3 or >= 9 bases and an N2 that runs past the end reject the row;
-//   set_barcode (:281-326): N1 + N2, a short N1 padded with 'S' (quality '?'), a long one cut to five bases + 'L';
-//   check_umi_quality (:340-352): more than `max_below` bases under `min_q`, or a mean under `avg_q`, rejects the row.
+// What collapse.py does per row before any grouping (get_barcode_positions, collapse.py:367-479): an 'N' anywhere rejects
+// the row (unless -N); spacer 1 is searched in its window bc[lo:hi] and must be found exactly once (regex.findall:
+// leftmost, non-overlapping).  Then, per layout of the ligation oligo:
+//   two spacers (M13, I8): window bc[0 : 10 + len(spacer1)]; spacer 2 is searched in bc[len(spacer1):] and must be found
+//     exactly once; N1 lies between the spacers, N2 is the six bases behind spacer 2;
+//   N1, spacer, N2 (I8_single): window bc[0:18]; N1 is bc[0 : spacer position], N2 the six bases behind the spacer;
+//     for both: N1 of <= 3 or >= 9 bases and an N2 that runs past the end reject the row, and set_barcode (:281-326)
+//     makes N1 + N2, a short N1 padded with 'S' (quality '?'), a long one cut to five bases + 'L';
+//   fixed barcode (NEBIO: window bc[18:28], barcode bc[0:17]; TAKARA: window bc[0:19], barcode bc[0:12]): the spacer only
+//     has to be there, its position is not used.
+// check_umi_quality (:340-352): more than `max_below` barcode qualities under `min_q`, or a mean under `avg_q`, rejects the row.
 // Only the EXACT spacer search is done here.  The reference escalates to fuzzy regular expressions ({1s<=2}, then
 // {2i+2d+1s<=2}) when an exact search finds nothing: such rows (a few percent) come back as DCB_BC_HOST and the host
-// runs the reference's own search on them; so do rows with symbols outside ACGTN or a quality string of another length.
+// runs the reference's own search on them; so do rows with symbols outside ACGTN, a quality string of another length, a
+// region longer than 250, and fixed-barcode regions shorter than the barcode (the reference would cut the barcode short).
 __device__ __forceinline__ int bc_find(const unsigned char* s, int from, int to, const char* pat, int plen) {   // first match in [from, to)
     for (int p = from; p + plen <= to; p++) {
         int k = 0;
@@ -313,7 +318,8 @@ __device__ __forceinline__ int bc_count(const unsigned char* s, int from, int to
     for (int p = bc_find(s, from, to, pat, plen); p >= 0; p = bc_find(s, p + plen, to, pat, plen)) { if (!n) first = p; n++; }
     return n;
 }
-struct BcParams { char sp1[32], sp2[32]; int len1, len2, allow_ns, min_q, max_below; double avg_q; };
+enum { BC_TWO_SPACERS = 0, BC_N1_SPACER_N2 = 1, BC_FIXED = 2 };   // BcParams::layout
+struct BcParams { char sp1[32], sp2[32]; int layout, lo, hi, bclen, len1, len2, allow_ns, min_q, max_below; double avg_q; };
 
 __global__ void __launch_bounds__(128)
 dcb_barcodes_kernel(const unsigned char* __restrict__ bc, const unsigned char* __restrict__ qual, const uint64_t* __restrict__ bc_off,
@@ -333,30 +339,39 @@ dcb_barcodes_kernel(const unsigned char* __restrict__ bc, const unsigned char* _
         odd |= !(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N');
     }
     if (has_n && !P.allow_ns) { status[i] = DCB_BC_FAIL_N; return; }                        // collapse.py:388-392
-    if (odd) return;
+    if (odd || (P.layout == BC_FIXED && L < P.bclen)) return;
     int w0, w1;
-    const int hi = L < 10 + P.len1 ? L : 10 + P.len1;
-    const int c1 = bc_count(s, 0, hi, P.sp1, P.len1, w0);                                   // :405-413
+    const int hi = L < P.hi ? L : P.hi;
+    const int c1 = bc_count(s, P.lo, hi, P.sp1, P.len1, w0);                                // :405-413
     if (c1 == 0) return;                                                                    // the fuzzy searches decide
     if (c1 != 1) { status[i] = DCB_BC_FAIL_NOSPACER; return; }
-    const int c2 = bc_count(s, P.len1, L, P.sp2, P.len2, w1);                               // :417-422
-    if (c2 == 0) return;
-    if (c2 != 1) { status[i] = DCB_BC_FAIL_NOT2; return; }
-    const int b1s = w0 + P.len1, b1e = w1, b2s = w1 + P.len2, b2e = b2s + 6, n1 = b1e - b1s;
-    if (n1 <= 3) { status[i] = DCB_BC_FAIL_N1SHORT; return; }                               // :241-254
-    if (n1 >= 9) { status[i] = DCB_BC_FAIL_N1LONG; return; }
-    if (b2e > L) { status[i] = DCB_BC_FAIL_N2END; return; }
-    n1len[i] = (uint8_t)n1;
-    // the 12 symbols (A C G T N S L = 0..6) and their qualities; a long N1 has no pad quality (11 values)
-    uint64_t cd = 12ull << 58;
+    // the barcode symbols (A C G T N S L = 0..6) and their qualities
+    uint64_t cd = (uint64_t)P.bclen << 58;
     int qsum = 0, qn = 0, below = 0, k = 0;
     auto sym = [](unsigned char c) -> uint64_t { return c == 'A' ? 0 : c == 'C' ? 1 : c == 'G' ? 2 : c == 'T' ? 3 : 4; };
     auto addq = [&](int v) { qsum += v; qn++; below += v < P.min_q; };
-    const int take1 = n1 > 6 ? 5 : n1;
-    for (int p = 0; p < take1; p++, k++) { cd |= sym(s[b1s + p]) << (3 * k); addq((int)q[b1s + p] - 33); }
-    if (n1 < 6) for (int p = n1; p < 6; p++, k++) { cd |= 5ull << (3 * k); addq('?' - 33); }   // 'S', quality '?'
-    if (n1 > 6) { cd |= 6ull << (3 * k); k++; }                                               // 'L'; "?" * (6 - n1) is empty
-    for (int p = 0; p < 6; p++, k++) { cd |= sym(s[b2s + p]) << (3 * k); addq((int)q[b2s + p] - 33); }
+    if (P.layout == BC_FIXED) {                                                             // set_barcode: bc[0:bclen], q[0:bclen]
+        for (; k < P.bclen; k++) { cd |= sym(s[k]) << (3 * k); addq((int)q[k] - 33); }
+    } else {
+        int b1s = 0, b1e = w0, b2s = w0 + P.len1;                                           // I8_single: N1, spacer, N2
+        if (P.layout == BC_TWO_SPACERS) {
+            const int c2 = bc_count(s, P.len1, L, P.sp2, P.len2, w1);                       // :417-422
+            if (c2 == 0) return;
+            if (c2 != 1) { status[i] = DCB_BC_FAIL_NOT2; return; }
+            b1s = w0 + P.len1; b1e = w1; b2s = w1 + P.len2;
+        }
+        const int b2e = b2s + 6, n1 = b1e - b1s;
+        if (n1 <= 3) { status[i] = DCB_BC_FAIL_N1SHORT; return; }                           // :241-254
+        if (n1 >= 9) { status[i] = DCB_BC_FAIL_N1LONG; return; }
+        if (b2e > L) { status[i] = DCB_BC_FAIL_N2END; return; }
+        n1len[i] = (uint8_t)n1;
+        // 12 symbols; a long N1 has no pad quality (11 values)
+        const int take1 = n1 > 6 ? 5 : n1;
+        for (int p = 0; p < take1; p++, k++) { cd |= sym(s[b1s + p]) << (3 * k); addq((int)q[b1s + p] - 33); }
+        if (n1 < 6) for (int p = n1; p < 6; p++, k++) { cd |= 5ull << (3 * k); addq('?' - 33); }   // 'S', quality '?'
+        if (n1 > 6) { cd |= 6ull << (3 * k); k++; }                                               // 'L'; "?" * (6 - n1) is empty
+        for (int p = 0; p < 6; p++, k++) { cd |= sym(s[b2s + p]) << (3 * k); addq((int)q[b2s + p] - 33); }
+    }
     code[i] = cd;
     const bool bad_q = below > P.max_below || (double)qsum / (double)qn < P.avg_q;            // :350-352
     status[i] = bad_q ? DCB_BC_FAIL_QUALITY : DCB_BC_OK;
@@ -626,11 +641,18 @@ int dcb_barcodes(dcb_dist* d, const char* bc_text, const uint64_t* bc_off, const
     if (n == 0) return DCB_OK;
     BcParams P;
     std::memset(&P, 0, sizeof(P));
-    const char *sp1, *sp2;
-    if (prm->oligo == DCB_OLIGO_M13) { sp1 = "GTCGTGACTGGGAAAACCCTGG"; sp2 = "GTCGTGAT"; }     // collapse.py:176-177
-    else if (prm->oligo == DCB_OLIGO_I8) { sp1 = "GTCGTGAT"; sp2 = "GTCGTGAT"; }
-    else { dcb_set_error("dcb_barcodes: oligo %d has no device path (M13 and I8 do)", prm->oligo); return DCB_EUNSUPPORTED; }
+    // spacers, window of spacer 1 and barcode length per design (collapse.py:172-189, 367-479)
+    const char *sp1, *sp2 = "";
+    switch (prm->oligo) {
+    case DCB_OLIGO_M13:       sp1 = "GTCGTGACTGGGAAAACCCTGG"; sp2 = "GTCGTGAT"; P.layout = BC_TWO_SPACERS; break;
+    case DCB_OLIGO_I8:        sp1 = "GTCGTGAT"; sp2 = "GTCGTGAT"; P.layout = BC_TWO_SPACERS; break;
+    case DCB_OLIGO_I8_SINGLE: sp1 = "ATCACGAC"; P.layout = BC_N1_SPACER_N2; break;
+    case DCB_OLIGO_NEBIO:     sp1 = "TACGGG"; P.layout = BC_FIXED; P.lo = 18; P.hi = 28; P.bclen = 17; break;
+    case DCB_OLIGO_TAKARA:    sp1 = "GTACGGG"; P.layout = BC_FIXED; P.lo = 0; P.hi = 19; P.bclen = 12; break;
+    default: dcb_set_error("dcb_barcodes: oligo %d has no device path (DCB_OLIGO_* are 0..4)", prm->oligo); return DCB_EUNSUPPORTED;
+    }
     P.len1 = (int)std::strlen(sp1); P.len2 = (int)std::strlen(sp2);
+    if (P.layout != BC_FIXED) { P.lo = 0; P.hi = 10 + P.len1; P.bclen = 12; }
     std::memcpy(P.sp1, sp1, P.len1); std::memcpy(P.sp2, sp2, P.len2);
     P.allow_ns = prm->allow_ns; P.min_q = prm->min_q; P.max_below = prm->max_below; P.avg_q = prm->avg_q;
     CUDA_TRY(cudaSetDevice(d->device));

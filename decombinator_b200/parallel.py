@@ -89,7 +89,7 @@ def all_to_all_bytes(chunks):
 
 # ---------------------------------------------------------------------------------------------------------
 # The collapse exchange: 64-byte records (SURVEY.md 8(d)), one NCCL all-to-all straight from device buffers.
-#   u64 global row index | u64 barcode (12 symbols x 3 bits over ACGTNSL, length in the top bits: what dcb_umi_pairs takes)
+#   u64 global row index | u64 barcode (up to 19 symbols x 3 bits over ACGTNSL, length in the top bits: what dcb_umi_pairs takes)
 #   u8 v, u8 j, u16 vdel, u16 jdel | u8 inter-tag length, u8 insert offset in it, u8 insert length, u8 flags
 #   33 B inter-tag sequence, 2 bits per base (<= 132 nt; -ln defaults to 130) | 5 B padding
 # The barcode was located and quality-filtered on the source rank, so the 42-nt barcode region, the quality strings and

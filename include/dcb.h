@@ -335,19 +335,24 @@ int dcb_lev_leq(dcb_dist*, const uint8_t* symbols, const uint64_t* off, const ui
  * alphabet); the pattern then takes eight bit planes instead of three. */
 int dcb_lev_leq_bytes(dcb_dist*, const uint8_t* symbols, const uint64_t* off, const uint32_t* len, uint32_t n_seqs,
                       const uint32_t* a, const uint32_t* b, uint64_t n_pairs, double frac, uint8_t* verdict);
-/* Barcode extraction of the collapse step, per decombined row: replaces, for the two-spacer oligos M13 and I8 and rows whose
- * spacers are found EXACTLY, get_barcode_positions (collapse.py:367-479), set_barcode (:281-326) and check_umi_quality
- * (:340-352).  bc / q: the barcode region of the row (field 8 of an .n12 row) and its quality string (field 9), as
- * (offset, length) into two text buffers.  Per row:
- *   status  DCB_BC_OK, the failure the reference would count (DCB_BC_FAIL_*), or DCB_BC_HOST: an exact spacer search found
- *           nothing, so the reference's fuzzy regular-expression searches decide (or the row has a symbol outside ACGTN / a
- *           quality string of another length): the caller runs the reference's own code on these rows;
- *   n1len   length of N1 (4..8) once the spacers are placed (also for DCB_BC_FAIL_QUALITY): 6 = plain, < 6 padded with 'S',
- *           > 6 cut to five bases + 'L' (the readdata_short_barcode / readdata_long_barcode counters);
- *   code    the 12-symbol barcode as dcb_umi_pairs takes it: 3 bits per symbol, A C G T N S L = 0..6, length in bits [58, 64). */
+/* Barcode extraction of the collapse step, per decombined row: replaces, for rows whose spacers are found EXACTLY,
+ * get_barcode_positions (collapse.py:367-479), set_barcode (:281-326) and check_umi_quality (:340-352), for every
+ * ligation-oligo design of -ol.  bc / q: the barcode region of the row (field 8 of an .n12 row) and its quality string
+ * (field 9), as (offset, length) into two text buffers.  Per row:
+ *   status  DCB_BC_OK, the failure the reference would count (DCB_BC_FAIL_*), or DCB_BC_HOST: an exact search of spacer 1
+ *           in its window (or of spacer 2) found nothing, so the reference's fuzzy regular-expression searches decide; so
+ *           also for a symbol outside ACGTN, a quality string of another length, a region longer than 250, and (TAKARA) a
+ *           region shorter than the 12-symbol barcode: the caller runs the reference's own code on these rows.
+ *           M13, I8: any DCB_BC_FAIL_*; I8_single: all but DCB_BC_FAIL_NOT2; NEBIO, TAKARA: DCB_BC_FAIL_N,
+ *           DCB_BC_FAIL_NOSPACER (two or more exact hits in the window) and DCB_BC_FAIL_QUALITY;
+ *   n1len   M13, I8, I8_single: length of N1 (4..8) once the spacers are placed (also for DCB_BC_FAIL_QUALITY): 6 = plain,
+ *           < 6 padded with 'S', > 6 cut to five bases + 'L' (the readdata_short_barcode / readdata_long_barcode
+ *           counters); NEBIO, TAKARA: 0 (no N1);
+ *   code    the barcode as dcb_umi_pairs takes it: 3 bits per symbol, A C G T N S L = 0..6, length in bits [58, 64):
+ *           N1 + N2 in 12 symbols (M13, I8, I8_single), bc[0:17] (NEBIO), bc[0:12] (TAKARA). */
 enum { DCB_BC_OK = 0, DCB_BC_FAIL_N = 1, DCB_BC_FAIL_NOSPACER = 2, DCB_BC_FAIL_NOT2 = 3, DCB_BC_FAIL_N1SHORT = 4, DCB_BC_FAIL_N1LONG = 5,
        DCB_BC_FAIL_N2END = 6, DCB_BC_FAIL_QUALITY = 7, DCB_BC_HOST = 255 };
-enum { DCB_OLIGO_M13 = 0, DCB_OLIGO_I8 = 1 };
+enum { DCB_OLIGO_M13 = 0, DCB_OLIGO_I8 = 1, DCB_OLIGO_I8_SINGLE = 2, DCB_OLIGO_NEBIO = 3, DCB_OLIGO_TAKARA = 4 };   /* other values: DCB_EUNSUPPORTED */
 typedef struct dcb_bc_params {
     int32_t oligo;       /* DCB_OLIGO_* (inputargs["oligo"]) */
     int32_t allow_ns;    /* inputargs["allowNs"] */

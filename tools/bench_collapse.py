@@ -1,8 +1,10 @@
 #!/usr/bin/env python
-"""Throughput of the collapse distance primitives (SURVEY 8(d)): pair verifications/s of dcb_umi_pairs and
-verdicts/s of dcb_lev_leq on synthetic inputs shaped like configs[3] (12-nt UMIs, <= 130-nt inter-tag sequences).
+"""Throughput of the collapse primitives (SURVEY 8(d)): pair verifications/s of dcb_umi_pairs and verdicts/s of
+dcb_lev_leq on synthetic inputs shaped like configs[3] (12-nt UMIs, <= 130-nt inter-tag sequences), and rows/s of
+dcb_barcodes for each ligation-oligo design on 42-nt barcode regions (the generator's read 2 with 0.5 % substitutions,
+re-laid out per design by tests/oligo_layouts.py).
 
-    python tools/bench_collapse.py [--umis 200000] [--pairs 2000000]     (GPU box)
+    python tools/bench_collapse.py [--umis 200000] [--pairs 2000000] [--barcode-rows 10000000]     (GPU box)
 
 Prints one JSON line; device times come from the library's own CUDA events (dcb_dist_last_ms)."""
 import argparse
@@ -13,6 +15,7 @@ import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import numpy as np  # noqa: E402
 
@@ -22,6 +25,7 @@ def main():
     ap.add_argument("--umis", type=int, default=200_000)
     ap.add_argument("--pairs", type=int, default=2_000_000)
     ap.add_argument("--big", type=int, default=2_000_000, help="UMIs of the configs[3]-scale pair search (0 = skip)")
+    ap.add_argument("--barcode-rows", type=int, default=10_000_000, help="barcode regions per design for dcb_barcodes (0 = skip)")
     args = ap.parse_args()
     from decombinator_b200 import _lib
     rng = np.random.default_rng(20260004)
@@ -78,13 +82,39 @@ def main():
     verdict = d.lev_leq(sym, off, lens, a, b, 0.1)
     wall_lev = time.perf_counter() - t0
     ms_lev = d.last_ms()
+    barcodes = bench_barcodes(d, args.barcode_rows) if args.barcode_rows else None
     print(json.dumps({
         "umi_pairs": {"unique_umis": U, "pairs_found": int(len(row)), "method": method, "device_ms": ms_pairs, "wall_s": wall_pairs,
                       "all_pairs_sweep": {"pair_checks": checks, "device_ms": ms_ap, "checks_per_s": checks / (ms_ap / 1e3)},
                       "algorithmic_bytes": 8 * U + 8 * int(len(row)), "hbm_GBps": (8 * U + 8 * len(row)) / (ms_pairs / 1e3) / 1e9},
         "umi_pairs_2M": big,
         "lev_leq": {"pairs": int(args.pairs), "accepted": int(verdict.sum()), "device_ms": ms_lev,
-                    "verdicts_per_s": args.pairs / (ms_lev / 1e3), "wall_s": wall_lev}}))
+                    "verdicts_per_s": args.pairs / (ms_lev / 1e3), "wall_s": wall_lev},
+        "barcodes": barcodes}))
+
+
+def bench_barcodes(d, n):
+    """dcb_barcodes over n 42-nt barcode regions per design, quality all 'I', -N off, the default quality filter."""
+    import oligo_layouts
+    from decombinator_b200 import _lib, tags
+    info = tags.load("human", "extended", "b")
+    syn = _lib.Synth([(info.v_regions, info.j_regions)], 20260004, 250, 62, 0.0, 0.0, 0.0, umi_pool=max(1000, n // 50),
+                     sub_rate2=0.005)
+    step = 1_000_000
+    r2 = np.concatenate([syn.reads(lo, min(step, n - lo), want_r2=True)[1].reshape(-1, 62) for lo in range(0, n, step)])
+    bo = np.arange(n, dtype=np.uint64) * np.uint64(62)
+    bl = np.full(n, 42, dtype=np.uint32)
+    qbuf, qo = np.full(64, ord("I"), dtype=np.uint8), np.zeros(n, dtype=np.uint64)
+    out = {"rows": n, "region": "42 nt of a 62-nt read 2, 0.5 % substitutions"}
+    for oligo in ("M13", "I8", "I8_single", "NEBIO", "TAKARA"):
+        text = np.ascontiguousarray(r2 if oligo == "M13" else oligo_layouts.relayout_array(r2, oligo)).reshape(-1)
+        code = _lib.OLIGOS_ON_DEVICE[oligo.lower()]
+        d.barcodes_arrays(text, bo[:1000], bl[:1000], qbuf, qo[:1000], bl[:1000], code, False, 20, 1, 30)
+        st, _, _ = d.barcodes_arrays(text, bo, bl, qbuf, qo, bl, code, False, 20, 1, 30)
+        ms = d.last_ms()
+        out[oligo] = {"device_ms": ms, "rows_per_s": n / (ms / 1e3), "decided_on_device": float((st != _lib.BC_HOST).mean()),
+                      "passed": float((st == _lib.BC_OK).mean())}
+    return out
 
 
 if __name__ == "__main__":

@@ -2,9 +2,12 @@
 """User-facing path from FASTQ text: `decombinator(inputargs)` on a synthetic paired FASTQ (GPU box only).
 
     python tools/e2e_fastq.py [--reads 2000000] [--python-fastq]
+    python tools/e2e_fastq.py --pipeline [--oligo I8_single|NEBIO|TAKARA]
 
 Writes R1/R2 files of the configs[1] recipe under /tmp, runs the drop-in stage function (decombine.py:881 of the
-reference) and prints where the wall time goes: ingest (FASTQ text -> record index), pack, device, row assembly.
+reference) and prints where the wall time goes: ingest (FASTQ text -> record index), pack, device, row assembly.  With --pipeline --oligo, read 2 is re-laid out for that ligation-oligo design
+(tests/oligo_layouts.py) and `pipeline` runs twice: as shipped, and with the barcodes of that design located on the
+host (the device path restricted to M13 and I8 in this process, as before the device took the other designs).
 """
 import argparse
 import json
@@ -14,6 +17,7 @@ import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import numpy as np  # noqa: E402
 
@@ -26,6 +30,8 @@ def main():
     ap.add_argument("--rows-as-text", action="store_true", help="what the `decombine` command does: rows handed over as .n12 text")
     ap.add_argument("--profile", action="store_true", help="cProfile of the timed decombinator() call")
     ap.add_argument("--pipeline", action="store_true", help="decombine + collapse (pipeline.run) on reads with repeated UMIs")
+    ap.add_argument("--oligo", default="M13", choices=["M13", "I8", "I8_single", "NEBIO", "TAKARA"],
+                    help="with --pipeline: read 2 laid out for this ligation-oligo design")
     args = ap.parse_args()
     from decombinator_b200 import _lib, decombine, fastq, io, tags
     info = tags.load("human", "extended", "b")
@@ -33,6 +39,9 @@ def main():
     syn = _lib.Synth([(info.v_regions, info.j_regions)], 20260002, L, 42 + 20, 0.0, 0.0, 0.0,
                      umi_pool=(max(1000, n // 20) if args.pipeline else 0))
     r1, r2 = syn.reads(0, n, want_r2=True)
+    if args.oligo != "M13":
+        import oligo_layouts
+        r2 = oligo_layouts.relayout_array(r2.reshape(n, 62), args.oligo).reshape(-1)
     os.makedirs("/tmp/e2e", exist_ok=True)
     p1, p2 = "/tmp/e2e/syn_1.fq", "/tmp/e2e/syn_2.fq"
     t0 = time.perf_counter()
@@ -62,7 +71,7 @@ def main():
     ia["rows_as_text"] = args.rows_as_text
     if args.pipeline:
         from decombinator_b200 import pipeline
-        ia.update(dontsave=True, oligo="M13", command="pipeline")
+        ia.update(dontsave=True, oligo=args.oligo, command="pipeline")
         t0 = time.perf_counter()
         rows = decombine.decombinator(dict(ia))
         t_dec = time.perf_counter() - t0
@@ -76,8 +85,18 @@ def main():
         if args.profile:
             pr.disable()
             pstats.Stats(pr).sort_stats("cumulative").print_stats(28)
-        print(json.dumps({"reads": n, "decombinator_s": round(t_dec, 2), "pipeline_s": round(t_pipe, 2), "rows": len(rows),
-                          "translated": len(out), "pipeline_reads_per_s": round(n / t_pipe)}))
+        line = {"reads": n, "oligo": args.oligo, "decombinator_s": round(t_dec, 2), "pipeline_s": round(t_pipe, 2), "rows": len(rows),
+                "translated": len(out), "pipeline_reads_per_s": round(n / t_pipe)}
+        if args.oligo.lower() not in ("m13", "i8"):
+            from decombinator_b200 import collapse
+            device_counts = dict(collapse.counts)
+            _lib.OLIGOS_ON_DEVICE = {"m13": 0, "i8": 1}          # this process only: the barcodes of args.oligo on the host
+            t0 = time.perf_counter()
+            host = pipeline.run(dict(ia))
+            t_host = time.perf_counter() - t0
+            same = host.equals(out) and all(collapse.counts[k] == v for k, v in device_counts.items() if isinstance(v, int) and not k.startswith("time_"))
+            line.update(host_barcodes_pipeline_s=round(t_host, 2), host_barcodes_pipeline_reads_per_s=round(n / t_host), same_output=bool(same))
+        print(json.dumps(line))
         return
     # warm-up: tables, context, CUDA
     small = dict(ia)
