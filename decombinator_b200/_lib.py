@@ -156,6 +156,12 @@ def lib():
     L.dcb_dist_last_ms.argtypes = [vp, ctypes.POINTER(ctypes.c_double)]
     L.dcb_dist_last_method.argtypes = [vp]
     L.dcb_dist_last_method.restype = ctypes.c_char_p
+    L.dcb_translate_tables_build.argtypes = [i32, cpp, cpp, vp, cpp, cpp, cpp, i32, cpp, cpp, vp, cpp, ctypes.POINTER(ctypes.c_void_p)]
+    L.dcb_translate_tables_free.argtypes = [vp]
+    L.dcb_translate_tables_free.restype = None
+    L.dcb_translate_tables_blob.argtypes = [vp, ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_size_t)]
+    L.dcb_translate.argtypes = [vp, vp, vp, u64] + [vp] * 10 + [u64, i32, i32, vp, vp, ctypes.POINTER(u64),
+                                ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(u64)]
     L.dcb_synth_create.restype = vp
     L.dcb_synth_create.argtypes = [ctypes.POINTER(CSynthParams), i32, ctypes.POINTER(cpp), ctypes.POINTER(ctypes.c_int),
                                    ctypes.POINTER(cpp), ctypes.POINTER(ctypes.c_int)]
@@ -874,6 +880,73 @@ def encode_seqs(seqs):
         off[1:] = np.cumsum(length[:-1], dtype=np.uint64)
     raw = np.frombuffer("".join(seqs).encode("latin-1"), dtype=np.uint8)
     return table[raw], off, length
+
+
+class TranslateTables:
+    """dcb_translate_tables: the germline tables of one chain for dcb_translate.  Raises DcbError (code in .rc) when
+    the tables are outside what the kernels take (DCB_EUNSUPPORTED: e.g. a J motif other than four capitals or '.')."""
+
+    def __init__(self, v_regions, v_calls, v_pos, v_residue, v_cdr1, v_cdr2, j_regions, j_calls, j_pos, j_motif):
+        L = lib()
+        nv, nj = len(v_regions), len(j_regions)
+        self._keep = [_carr(x) for x in (v_regions, v_calls, v_residue, v_cdr1, v_cdr2, j_regions, j_calls, j_motif)]
+        vp_, jp_ = np.ascontiguousarray(v_pos, dtype=np.int32), np.ascontiguousarray(j_pos, dtype=np.int32)
+        k = self._keep
+        out = ctypes.c_void_p()
+        rc = L.dcb_translate_tables_build(nv, k[0], k[1], vp_.ctypes.data, k[2], k[3], k[4], nj, k[5], k[6], jp_.ctypes.data, k[7],
+                                          ctypes.byref(out))
+        self._h = out.value
+        if rc != 0:
+            err = DcbError("dcb_translate_tables_build failed (%d): %s" % (rc, L.dcb_last_error().decode()))
+            err.rc = rc
+            raise err
+
+    def blob(self):
+        p, n = ctypes.c_void_p(), ctypes.c_size_t()
+        _check(lib().dcb_translate_tables_blob(self._h, ctypes.byref(p), ctypes.byref(n)), "dcb_translate_tables_blob")
+        return np.frombuffer((ctypes.c_uint8 * n.value).from_address(p.value), dtype=np.uint8).copy()
+
+    def __del__(self):
+        try:
+            if self._h:
+                lib().dcb_translate_tables_free(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+
+class PinnedText(NativeText):
+    """Page-locked text returned by dcb_translate; freed with dcb_pinned_free."""
+
+    def __del__(self):
+        try:
+            if self._p:
+                self.a = None
+                lib().dcb_pinned_free(self._p)
+                self._p = None
+        except Exception:
+            pass
+
+
+TR_SYMBOL, TR_GENE, TR_CINDEX, TR_QUOTE, TR_LONG = 1, 2, 4, 8, 16
+
+
+def translate_rows(dist, tables, text, v, j, vdel, jdel, id_off, id_len, ins_off, ins_len, freq, cluster, npf, nbc):
+    """dcb_translate over rows given as columns (dist: a Dist, or None to ask the library without a context).
+    -> (text or None when rows are flagged, productive bool array, row flags uint8 array)."""
+    n = len(v)
+    u32 = lambda a: np.ascontiguousarray(a, dtype=np.uint32)
+    u64 = lambda a: np.ascontiguousarray(a, dtype=np.uint64)
+    i64 = lambda a: np.ascontiguousarray(a, dtype=np.int64)
+    cols = [u32(v), u32(j), u32(vdel), u32(jdel), u64(id_off), u32(id_len), u64(ins_off), u32(ins_len), i64(freq), i64(cluster)]
+    buf = np.frombuffer(text, dtype=np.uint8) if not isinstance(text, np.ndarray) else text
+    prod, flags = np.zeros(n, dtype=np.uint8), np.zeros(n, dtype=np.uint8)
+    nf, out, nb = ctypes.c_uint64(), ctypes.c_void_p(), ctypes.c_uint64()
+    _check(lib().dcb_translate(dist._h if dist is not None else None, tables._h, buf.ctypes.data if len(buf) else None, len(buf),
+                               *[c.ctypes.data for c in cols], n, int(bool(npf)), int(bool(nbc)), prod.ctypes.data, flags.ctypes.data,
+                               ctypes.byref(nf), ctypes.byref(out), ctypes.byref(nb)), "dcb_translate")
+    body = PinnedText(out.value, nb.value) if out.value else (b"" if nf.value == 0 else None)
+    return body, prod.astype(bool), flags
 
 
 class Dist:

@@ -18,7 +18,7 @@ VARIANT_DIR = os.path.join(os.path.dirname(HERE), "build")
 SYNTH_LIB = os.path.join(HERE, "libdcbsynth.so")   # the synthetic read generator alone (bench.py's reference arm maps only this + oracle/)
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 
-SOURCES = ["decombine.cu", "collapse.cu", "tagset.cpp", "pack.cpp", "fastq.cpp", "group.cpp", "synth.cpp", "error.cpp"]
+SOURCES = ["decombine.cu", "collapse.cu", "translate.cu", "tagset.cpp", "pack.cpp", "fastq.cpp", "group.cpp", "synth.cpp", "error.cpp"]
 
 FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

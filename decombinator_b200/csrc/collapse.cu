@@ -688,6 +688,14 @@ int dcb_barcodes(dcb_dist* d, const char* bc_text, const uint64_t* bc_off, const
 
 const char* dcb_dist_last_method(const dcb_dist* d) { return d ? d->last_method : ""; }
 
+}  // extern "C"
+
+int dcb_dist_device(const dcb_dist* d) { return d->device; }
+void* dcb_dist_stream(const dcb_dist* d) { return (void*)d->stream; }
+void dcb_dist_set_last_ms(dcb_dist* d, double ms) { d->last_ms = ms; }
+
+extern "C" {
+
 int dcb_dist_last_ms(dcb_dist* d, double* ms) {
     if (!d || !ms) return DCB_EINVAL;
     *ms = d->last_ms;

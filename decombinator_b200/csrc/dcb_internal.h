@@ -28,6 +28,11 @@ extern "C" int dcb_packed_alloc(uint64_t n, uint32_t slot_words, uint32_t n_exc,
 extern "C" int dcb_pack_words(const char* ascii, const uint64_t* off, const uint32_t* len, uint64_t first, uint64_t count, uint32_t uniform_len,
                               int revcomp, uint32_t slot_words, uint32_t* words, int n_threads, int* clean);
 
+// The light context of collapse.cu, for the other entry points that hang off it (translate.cu).
+int dcb_dist_device(const dcb_dist* d);
+void* dcb_dist_stream(const dcb_dist* d);
+void dcb_dist_set_last_ms(dcb_dist* d, double ms);
+
 #if defined(__GNUC__)
 __attribute__((format(printf, 1, 2)))
 #endif

@@ -146,14 +146,19 @@ def write_out_intermediate(data: list, inputargs: dict, suffix: str):
 
 
 def write_out_translated(data, inputargs: dict):
-    """AIRR ``.tsv`` writer: ``DataFrame.to_csv(sep="\\t", index=False)``, gzip unless -dz (io.py:516-548)."""
+    """AIRR ``.tsv`` writer: ``DataFrame.to_csv(sep="\\t", index=False)``, gzip unless -dz (io.py:516-548).  `data`: the
+    DataFrame of cdr3translator, or the text of translate.translate_tsv (written as it is: the same bytes)."""
     chainnams = {"a": "alpha", "b": "beta", "g": "gamma", "d": "delta"}
     filename_id = os.path.basename(inputargs["infile"]).split(".")[0]
     if inputargs["command"] in ["collapse", "translate"]:
         outfilename = inputargs["outpath"] + f"{filename_id}" + ".tsv"
     else:
         outfilename = inputargs["outpath"] + inputargs["prefix"] + f"{filename_id}" + f"_{chainnams[inputargs['chain'].lower()]}" + ".tsv"
-    data.to_csv(f"{outfilename}", sep="\t", index=False)
+    if hasattr(data, "to_csv"):
+        data.to_csv(f"{outfilename}", sep="\t", index=False)
+    else:
+        with open(outfilename, "wb") as outfile:
+            data.write(outfile)
     if not inputargs["dontgzip"]:
         print("Compressing pipeline output file to", outfilename + ".gz")
         with open(outfilename) as infile, gzip.open(outfilename + ".gz", "wt") as outfile:

@@ -17,10 +17,16 @@ def _world():
 def run(args=None, cli_args=None):
     """Decombine -> .n12 -> collapse -> .freq -> translate -> .tsv, stages chained in memory (reference pipeline.py:10-38).
     Returns the translated DataFrame (the reference returns nothing; its tests read the files)."""
+    return _run(cli_args if cli_args else args, frame=True)
+
+
+def _run(inputargs, frame):
+    """run(); frame=False (the command line): the translate stage hands its .tsv text straight to the writer, and no
+    DataFrame is built (nor pandas imported) unless a row needs the host path."""
     start = datetime.now()
-    inputargs = cli_args if cli_args else args
     from .collapse import collapsinator
-    from .translate import cdr3translator
+    from .translate import cdr3translator, translate_tsv
+    translator = cdr3translator if frame else translate_tsv
     if _world() > 1:
         from . import parallel
         rank, _ = parallel.init_from_env()
@@ -35,7 +41,7 @@ def run(args=None, cli_args=None):
         print("Collapsinator complete...")
         if rank != 0:
             return data
-        data = cdr3translator(data=data, inputargs=inputargs)     # the collapsed rows are few: rank 0 translates them
+        data = translator(data=data, inputargs=inputargs)     # the collapsed rows are few: rank 0 translates them
         print("CDR3translator complete...")
         if not inputargs["dontsave"]:
             write_out_translated(data, inputargs)
@@ -50,7 +56,7 @@ def run(args=None, cli_args=None):
     if not inputargs["dontsave"]:
         write_out_intermediate(data, inputargs, ".freq")
     print("Collapsinator complete...")
-    data = cdr3translator(data=data, inputargs=inputargs)
+    data = translator(data=data, inputargs=inputargs)
     print("CDR3translator complete...")
     if not inputargs["dontsave"]:
         write_out_translated(data, inputargs)
@@ -80,11 +86,11 @@ def main():
         if rank == 0:
             write_out_intermediate(data, inputargs, ".freq")
     elif inputargs["command"] == "translate":
-        from .translate import cdr3translator
-        if rank == 0:                                   # host-only stage over the collapsed rows: one process does it
-            write_out_translated(cdr3translator(inputargs=inputargs), inputargs)
+        from .translate import translate_tsv
+        if rank == 0:                                   # the collapsed rows are few: one process translates them
+            write_out_translated(translate_tsv(inputargs=inputargs), inputargs)
     else:
-        run(cli_args=inputargs)
+        _run(inputargs, frame=False)
 
 
 if __name__ == "__main__":

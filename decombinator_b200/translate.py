@@ -9,12 +9,16 @@ Same entry points and contracts as /root/reference/src/decombinator/translate.py
 * ``import_gene_information(inputargs)`` (translate.py:123-254) and ``get_cdr3(dcr, headers, inputargs)``
   (translate.py:257-357).
 
-This stage runs once per UNIQUE rearrangement of a sample (the collapsed output), so it is host code: the work per
-row is rebuilding the nucleotide sequence from the germline regions, translating it, and four string checks.  What is
-different from the reference is the structure (one ``GeneTables`` object instead of a dozen module globals, the
-translation of every (V gene, deletion) prefix cached because repertoires reuse them heavily) and that the translation
-itself is implemented here (Bio.Seq.translate's standard-table semantics) instead of importing Biopython, which GPU
-nodes do not carry.  Quirks kept on purpose, because the goldens depend on them or a user may:
+The work per row is rebuilding the nucleotide sequence from the germline regions, translating it, and four string
+checks.  When a CUDA device is usable, ``dcb_translate`` (csrc/translate.cu) does that for every row and writes the
+``.tsv`` lines itself; ``translate_tsv`` hands that text on without building a DataFrame (the command line writes it
+as it is).  The host code below -- ``get_cdr3`` and the loop of ``_translate_host`` -- is the path without a device,
+the path of a call with a row outside the kernels' envelope (``_lib.TR_*``: the host raises on it, or to_csv would
+quote it), and the reference the tests compare the kernels with.  What is different from the reference is the
+structure (one ``GeneTables`` object instead of a dozen module globals, the translation of every (V gene, deletion)
+prefix cached because repertoires reuse them heavily) and that the translation itself is implemented here
+(Bio.Seq.translate's standard-table semantics) instead of importing Biopython, which GPU nodes do not carry.  Quirks
+kept on purpose, because the goldens depend on them or a user may:
 
 * gene names are the second ``|`` field of the FASTA header, upper-cased, cut at ``*`` (translate.py:189-192, 293-294);
 * "functionality" is column 3 of the ``.translate`` file (translate.py:217-219) -- the gene name, not the F/ORF/P
@@ -31,14 +35,15 @@ import re
 import sys
 from time import strftime
 
-import pandas as pd
+import numpy as np
 
-from . import __version__, tags
+from . import __version__, _lib, tags
 
 chainnams = tags.CHAINNAMS
 counts = coll.Counter()
 chain = None
 _genes = None      # GeneTables of the last import_gene_information()
+_dist = None       # dcb_dist of this process; False when no device is usable
 
 out_headers = [
     "sequence_id", "v_call", "d_call", "j_call", "junction_aa", "duplicate_count", "sequence", "junction",
@@ -276,29 +281,188 @@ def _summary_file(logpath, stem):
     raise RuntimeError("no free summary file name")
 
 
-def cdr3translator(inputargs: dict, data=None) -> pd.DataFrame:
-    """Function wrapper for CDR3translator (translate.py:388-621)."""
-    global counts
-    counts = coll.Counter()
-    print("Running CDR3Translator version", __version__)
-    ch = _resolve_chain(inputargs)
-    inputargs["chain"] = ch          # the corrected value is what import_gene_information reads
-    import_gene_information(inputargs)
-    g = _genes
+def _device():
+    """The dcb_dist context the device path runs on, or None when no CUDA device is usable."""
+    global _dist
+    if _dist is None:
+        try:
+            _dist = _lib.Dist(device=int(os.environ.get("LOCAL_RANK", "0")))
+        except _lib.DcbError:
+            _dist = False
+    return _dist or None
 
+
+def device_tables(g):
+    """dcb_translate_tables of a GeneTables (built once per object), or None when the kernels cannot take this chain."""
+    if not hasattr(g, "_device_tables"):
+        g._device_tables = None
+        nv, nj = len(g.v_regions), len(g.j_regions)
+        if all(len(x) == nv for x in (g.v_names, g.v_translate_position, g.v_translate_residue, g.v_cdr1, g.v_cdr2)) and \
+                all(len(x) == nj for x in (g.j_names, g.j_translate_position, g.j_translate_residue)):
+            try:
+                g._device_tables = _lib.TranslateTables(
+                    g.v_regions, [n.split("*")[0] for n in g.v_names], g.v_translate_position, g.v_translate_residue, g.v_cdr1,
+                    g.v_cdr2, g.j_regions, [n.split("*")[0] for n in g.j_names], g.j_translate_position, g.j_translate_residue)
+            except (_lib.DcbError, UnicodeEncodeError):
+                pass
+    return g._device_tables
+
+
+_U32 = 0xFFFFFFFF
+
+
+def _parse_uints(buf, s, e):
+    """int() of the fields buf[s:e] when every field is optional spaces then 1..15 digits; None otherwise."""
+    n = len(s)
+    width = e - s
+    if n and (int(width.min()) < 1 or int(width.max()) > 16):
+        return None
+    val, seen = np.zeros(n, dtype=np.int64), np.zeros(n, dtype=bool)
+    for k in range(int(width.max()) if n else 0):
+        live = k < width
+        c = buf[np.where(live, s + k, 0)].astype(np.int64)
+        dig = live & (c >= 48) & (c <= 57)
+        space = live & (c == 32)
+        if (space & seen).any() or (live & ~dig & ~space).any():
+            return None
+        val = np.where(dig, val * 10 + (c - 48), val)
+        seen |= dig
+    return val if seen.all() else None
+
+
+def _columns_from_freq(raw):
+    """Columns of dcb_translate from .freq text (seven ',' separated fields per line), split as the host does:
+    decombinator_id = ",".join(fields[:5]) (fields keep their leading space), insert = fields[4][1:], int() of the rest.
+    None when the text is not plainly of that shape (the host path then reads it)."""
+    buf = np.frombuffer(raw, dtype=np.uint8)
+    if len(buf) == 0:
+        return dict(text=buf, n=0)
+    if (buf >= 0x80).any() or (buf == 13).any():        # decoding / universal newlines: the host's business
+        return None
+    ends = np.flatnonzero(buf == 10)
+    if buf[-1] != 10:
+        ends = np.append(ends, len(buf))
+    n = len(ends)
+    starts = np.empty(n, dtype=np.int64)
+    starts[0] = 0
+    starts[1:] = ends[:-1] + 1
+    commas = np.flatnonzero(buf == 44)
+    per_line = np.diff(np.searchsorted(commas, ends), prepend=0)
+    if len(commas) != 6 * n or (per_line != 6).any():
+        return None
+    c = commas.reshape(n, 6)
+    fs = [starts] + [c[:, k] + 1 for k in range(6)]
+    fe = [c[:, k] for k in range(6)] + [ends]
+    nums = {}
+    for k in (0, 1, 2, 3, 5, 6):
+        nums[k] = _parse_uints(buf, fs[k], fe[k])
+        if nums[k] is None:
+            return None
+    ins_off = fs[4] + 1
+    return dict(text=buf, n=n, v=nums[0], j=nums[1], vdel=nums[2], jdel=nums[3], freq=nums[5], cluster=nums[6],
+                id_off=starts, id_len=c[:, 4] - starts, ins_off=ins_off, ins_len=np.maximum(fe[4] - ins_off, 0))
+
+
+def _columns_from_rows(data):
+    """Columns of dcb_translate from collapsinator's rows ([v, j, vdel, jdel, insert] as str, count and cluster size as
+    int): decombinator_id = ", ".join(row[:5]).  None for rows of any other shape (the host path then takes them)."""
+    if not isinstance(data, list):
+        return None
+    n = len(data)
+    if n == 0:
+        return dict(text=np.zeros(0, dtype=np.uint8), n=0)
+    if any(len(r) != 7 for r in data):
+        return None
+    cols = list(zip(*data))
+    if not all(type(x) is str for k in range(5) for x in cols[k]) or not all(type(x) is int for k in (5, 6) for x in cols[k]):
+        return None
+    try:
+        nums = [np.fromiter(map(int, cols[k]), dtype=np.int64, count=n) for k in range(4)]
+        freq = np.fromiter(cols[5], dtype=np.int64, count=n)
+        cluster = np.fromiter(cols[6], dtype=np.int64, count=n)
+        ids = [", ".join(r[:5]) for r in data]
+        text = "\n".join(ids).encode("ascii")
+    except (ValueError, OverflowError, UnicodeEncodeError):        # the host path raises (or copes) as it always did
+        return None
+    if any((x < 0).any() for x in nums):
+        return None
+    id_len = np.fromiter(map(len, ids), dtype=np.int64, count=n)
+    id_off = np.zeros(n, dtype=np.int64)
+    np.cumsum(id_len[:-1] + 1, out=id_off[1:])
+    ins_len = np.fromiter(map(len, cols[4]), dtype=np.int64, count=n)
+    return dict(text=np.frombuffer(text, dtype=np.uint8), n=n, v=nums[0], j=nums[1], vdel=nums[2], jdel=nums[3], freq=freq,
+                cluster=cluster, id_off=id_off, id_len=id_len, ins_off=id_off + id_len - ins_len, ins_len=ins_len)
+
+
+class TsvText:
+    """The .tsv of a translate call as text: `header` + `body` (the kernels' lines, page-locked) -- what
+    DataFrame.to_csv(sep="\\t", index=False) of the call's DataFrame writes."""
+
+    def __init__(self, body, nobarcoding):
+        self.header = ("\t".join(out_headers) + "\n").encode()
+        self.body = body
+        self.nobarcoding = nobarcoding
+
+    def write(self, fh):
+        fh.write(self.header)
+        if len(self.body):
+            fh.write(memoryview(self.body.a) if hasattr(self.body, "a") else self.body)
+
+    def tobytes(self):
+        return self.header + bytes(self.body)
+
+    def frame(self):
+        """The DataFrame of the host path: str columns, duplicate_count int64, av_UMI_cluster_size int64 (or "")."""
+        import pandas as pd
+        lines = bytes(self.body).decode("ascii").split("\n")[:-1]
+        if not lines:
+            return pd.DataFrame([], columns=out_headers)
+        cols = dict(zip(out_headers, (list(c) for c in zip(*(line.split("\t") for line in lines)))))
+        cols["duplicate_count"] = list(map(int, cols["duplicate_count"]))
+        if not self.nobarcoding:
+            cols["av_UMI_cluster_size"] = list(map(int, cols["av_UMI_cluster_size"]))
+        return pd.DataFrame(cols, columns=out_headers)
+
+
+def _translate_device(inputargs, g, data):
+    """-> (TsvText, v, j, productive) or None when the host path must take the call."""
+    d = _device()
+    if d is None:
+        return None
+    tables = device_tables(g)
+    if tables is None:
+        return None
+    if inputargs["command"] == "translate":
+        opener = gzip.open if inputargs["infile"].endswith(".gz") else open
+        with opener(inputargs["infile"], "rb") as fh:
+            cols = _columns_from_freq(fh.read())
+    else:
+        cols = _columns_from_rows(data)
+    if cols is None:
+        return None
+    nbc = bool(inputargs["nobarcoding"])
+    if cols["n"] == 0:
+        z = np.zeros(0, dtype=np.int64)
+        return TsvText(b"", nbc), z, z, np.zeros(0, dtype=bool)
+    clip = lambda a: np.minimum(a, _U32)
+    body, productive, _ = _lib.translate_rows(d, tables, cols["text"], clip(cols["v"]), clip(cols["j"]), clip(cols["vdel"]),
+                                              clip(cols["jdel"]), cols["id_off"], cols["id_len"], cols["ins_off"], cols["ins_len"],
+                                              cols["freq"], cols["cluster"], inputargs["nonproductivefilter"], nbc)
+    if body is None:
+        return None
+    return TsvText(body, nbc), cols["v"], cols["j"], productive
+
+
+def _translate_host(inputargs, g, data):
+    """The row loop of the reference's CDR3translator (translate.py:430-540) -> (DataFrame, v, j, productive)."""
+    import pandas as pd
     from_file = inputargs["command"] == "translate"
     if from_file:
-        findfile(inputargs["infile"])
         opener = gzip.open if inputargs["infile"].endswith(".gz") else open
         infile = opener(inputargs["infile"], "rt")
     else:
         infile = data
-    counts["line_count"] = 0
-    print("Translating", chainnams[ch], "chain CDR3s from", inputargs["infile"])
-    filename_id = os.path.basename(inputargs["infile"]).split(".")[0]
-    count_functionality = inputargs["tags"] == "extended" and inputargs["species"] == "human"
-
-    rows = []
+    rows, vs, js, prod = [], [], [], []
     for line in infile:
         counts["line_count"] += 1
         if from_file:
@@ -323,23 +487,59 @@ def cdr3translator(inputargs: dict, data=None) -> pd.DataFrame:
         fields["sequence_id"] = str(counts["line_count"])
         fields["duplicate_count"] = frequency
         fields["av_UMI_cluster_size"] = cluster
-        if fields["productive"] == "T":
-            counts["prod_recomb"] += 1
-            tagp = "P"
+        productive = fields["productive"] == "T"
+        if productive or not inputargs["nonproductivefilter"]:
             rows.append([fields[h] for h in out_headers])
-        else:
-            counts["NP_count"] += 1
-            tagp = "NP"
-            if not inputargs["nonproductivefilter"]:
-                rows.append([fields[h] for h in out_headers])
-        if count_functionality:
-            counts[tagp + "_V-" + g.v_functionality[v]] += 1
-            counts[tagp + "_J-" + g.j_functionality[j]] += 1
+        vs.append(v)
+        js.append(j)
+        prod.append(productive)
     if from_file:
         infile.close()
-
     out_df = pd.DataFrame(rows, columns=out_headers)
     print("CDR3 data written to dataframe")
+    return out_df, vs, js, prod
+
+
+def translate_tsv(inputargs: dict, data=None):
+    """cdr3translator's work with the .tsv as text where a device is usable: -> TsvText, or the host path's
+    DataFrame when no device is usable or a row is outside the kernels' envelope.  Writes the summary like
+    cdr3translator.  Either result goes to io.write_out_translated."""
+    global counts
+    counts = coll.Counter()
+    print("Running CDR3Translator version", __version__)
+    ch = _resolve_chain(inputargs)
+    inputargs["chain"] = ch          # the corrected value is what import_gene_information reads
+    import_gene_information(inputargs)
+    g = _genes
+
+    if inputargs["command"] == "translate":
+        findfile(inputargs["infile"])
+    counts["line_count"] = 0
+    print("Translating", chainnams[ch], "chain CDR3s from", inputargs["infile"])
+    filename_id = os.path.basename(inputargs["infile"]).split(".")[0]
+    count_functionality = inputargs["tags"] == "extended" and inputargs["species"] == "human"
+
+    res = _translate_device(inputargs, g, data)
+    if res is not None:
+        print("CDR3 data translated on the GPU")
+    else:
+        res = _translate_host(inputargs, g, data)
+        counts = coll.Counter()                  # recounted from the columns below, as for the device path
+    out, v, j, productive = res
+    v, j, productive = np.asarray(v, dtype=np.int64), np.asarray(j, dtype=np.int64), np.asarray(productive, dtype=bool)
+    counts["line_count"] = len(productive)
+    n_prod = int(productive.sum())
+    if n_prod:
+        counts["prod_recomb"] = n_prod
+    if len(productive) - n_prod:
+        counts["NP_count"] = len(productive) - n_prod
+    if count_functionality:
+        for tagp, sel in (("P", productive), ("NP", ~productive)):
+            for gene, idx, func in (("V", v, g.v_functionality), ("J", j, g.j_functionality)):
+                idx = np.where(idx < 0, idx + len(func), idx)          # Python indexing of the host loop
+                for k, c in enumerate(np.bincount(idx[sel], minlength=len(func))):
+                    if c:
+                        counts[tagp + "_" + gene + "-" + func[k]] += int(c)
 
     if not inputargs["suppresssummary"]:
         logpath = inputargs["outpath"] + f"Logs{os.sep}"
@@ -364,4 +564,10 @@ def cdr3translator(inputargs: dict, data=None) -> pd.DataFrame:
         print(text, file=fh)
         fh.close()
         sort_permissions(summaryname)
-    return out_df
+    return out
+
+
+def cdr3translator(inputargs: dict, data=None) -> "pandas.DataFrame":
+    """Function wrapper for CDR3translator (translate.py:388-621)."""
+    out = translate_tsv(inputargs, data)
+    return out.frame() if isinstance(out, TsvText) else out

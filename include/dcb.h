@@ -364,8 +364,47 @@ int dcb_barcodes(dcb_dist*, const char* bc_text, const uint64_t* bc_off, const u
                  const uint64_t* q_off, const uint32_t* q_len, uint64_t n, const dcb_bc_params* prm, uint8_t* status,
                  uint8_t* n1len, uint64_t* code);
 
-/* Device time of the last dcb_umi_pairs (pair search, incl. its sorts on the deletion-neighbourhood path) or
-   dcb_lev_leq kernel (CUDA events). */
+/* ---------------------------------------------------------------------------------------------
+ * Translate stage: get_cdr3 (translate.py:257-357) for DCR rows and the AIRR .tsv line of each, as
+ * DataFrame.to_csv(sep="\t", index=False) writes it (io.py:516-548).
+ *
+ * Tables of one chain (host only, no GPU needed), from what import_gene_information reads
+ * (translate.py:123-254): per V gene the upper-cased region, the call (name cut at '*'), the conserved
+ * residue's position and residue, CDR1 / CDR2 ("" where there are none); per J gene the region, the call,
+ * the motif window start and the motif.  Motifs must be four symbols, each a capital letter or '.',
+ * regions upper-case IUPAC of at most 1024 bases, names and CDRs printable ASCII without '"'
+ * (DCB_EUNSUPPORTED otherwise: the caller keeps the host path).
+ * ------------------------------------------------------------------------------------------- */
+typedef struct dcb_translate_tables dcb_translate_tables;
+int dcb_translate_tables_build(int n_v, const char* const* v_regions, const char* const* v_calls, const int32_t* v_pos,
+                               const char* const* v_residue, const char* const* v_cdr1, const char* const* v_cdr2, int n_j,
+                               const char* const* j_regions, const char* const* j_calls, const int32_t* j_pos,
+                               const char* const* j_motif, dcb_translate_tables** out);
+void dcb_translate_tables_free(dcb_translate_tables*);
+/* The flattened blob the kernels stage in shared memory (tests compile csrc/translate_core.cuh over it). */
+int dcb_translate_tables_blob(const dcb_translate_tables*, const uint8_t** bytes, size_t* n_bytes);
+
+/* Row flags of dcb_translate: the row is outside the device path (the host would raise, or write it otherwise). */
+enum { DCB_TR_SYMBOL = 1,   /* an insert symbol outside IUPAC and U (either case) */
+       DCB_TR_GENE = 2,     /* v or j out of range */
+       DCB_TR_CINDEX = 4,   /* the conserved-C index lies beyond the protein */
+       DCB_TR_QUOTE = 8,    /* decombinator_id holds '"', a control or a non-ASCII byte (to_csv would quote or re-encode) */
+       DCB_TR_LONG = 16 };  /* the rebuilt sequence is longer than 1024 bases */
+
+/* n rows as columns.  decombinator_id of row i is text[id_off[i], + id_len[i]) (written verbatim), its insert
+ * text[ins_off[i], + ins_len[i]); freq / cluster: duplicate_count and av_UMI_cluster_size.  Row i is line
+ * sequence_id = i + 1.  nonproductive_filter (-npf) drops the lines of non-productive rows; nobarcoding (-nbc)
+ * writes duplicate_count 1 and an empty av_UMI_cluster_size.  Out: productive[i], row_flags[i] (DCB_TR_*),
+ * *n_flagged; when no row is flagged, *out is the text of the kept lines (no header) in page-locked memory
+ * (free with dcb_pinned_free), *out_bytes its size; with flagged rows *out is NULL.  d == NULL and no CUDA
+ * device: DCB_ENOGPU. */
+int dcb_translate(dcb_dist*, const dcb_translate_tables*, const char* text, uint64_t text_bytes, const uint32_t* v, const uint32_t* j,
+                  const uint32_t* vdel, const uint32_t* jdel, const uint64_t* id_off, const uint32_t* id_len, const uint64_t* ins_off,
+                  const uint32_t* ins_len, const int64_t* freq, const int64_t* cluster, uint64_t n, int nonproductive_filter,
+                  int nobarcoding, uint8_t* productive, uint8_t* row_flags, uint64_t* n_flagged, char** out, uint64_t* out_bytes);
+
+/* Device time of the last dcb_umi_pairs (pair search, incl. its sorts on the deletion-neighbourhood path),
+   dcb_lev_leq kernel or dcb_translate kernels and scan (CUDA events). */
 int dcb_dist_last_ms(dcb_dist*, double* ms);
 /* How the last dcb_umi_pairs searched: "deletion neighbourhoods" (max_edits <= 2 and a long list: what symdel does,
    collapse.py:735-740) or "all pairs" (short lists, max_edits > 2).  The environment variable DCB_UMI_SYMDEL_MIN moves

@@ -2,12 +2,14 @@
 """User-facing path from FASTQ text: `decombinator(inputargs)` on a synthetic paired FASTQ (GPU box only).
 
     python tools/e2e_fastq.py [--reads 2000000] [--python-fastq]
-    python tools/e2e_fastq.py --pipeline [--oligo I8_single|NEBIO|TAKARA]
+    python tools/e2e_fastq.py --pipeline [--oligo I8_single|NEBIO|TAKARA] [--cli]
 
 Writes R1/R2 files of the configs[1] recipe under /tmp, runs the drop-in stage function (decombine.py:881 of the
 reference) and prints where the wall time goes: ingest (FASTQ text -> record index), pack, device, row assembly.  With --pipeline --oligo, read 2 is re-laid out for that ligation-oligo design
 (tests/oligo_layouts.py) and `pipeline` runs twice: as shipped, and with the barcodes of that design located on the
-host (the device path restricted to M13 and I8 in this process, as before the device took the other designs).
+host (the device path restricted to M13 and I8 in this process, as before the device took the other designs).  With
+--pipeline --cli, `pipeline` runs as the command line runs it (the .n12, .freq and .tsv written with -dz, the translate
+stage handing its text to the writer), twice with the translate stage on the device and twice on the host, alternated.
 """
 import argparse
 import json
@@ -32,6 +34,7 @@ def main():
     ap.add_argument("--pipeline", action="store_true", help="decombine + collapse (pipeline.run) on reads with repeated UMIs")
     ap.add_argument("--oligo", default="M13", choices=["M13", "I8", "I8_single", "NEBIO", "TAKARA"],
                     help="with --pipeline: read 2 laid out for this ligation-oligo design")
+    ap.add_argument("--cli", action="store_true", help="with --pipeline: the command line's path, translate on the device and on the host")
     args = ap.parse_args()
     from decombinator_b200 import _lib, decombine, fastq, io, tags
     info = tags.load("human", "extended", "b")
@@ -75,6 +78,25 @@ def main():
         t0 = time.perf_counter()
         rows = decombine.decombinator(dict(ia))
         t_dec = time.perf_counter() - t0
+        if args.cli:
+            import hashlib
+            from decombinator_b200 import translate
+            ia.update(dontsave=False, dontgzip=True)
+            os.makedirs(ia["outpath"], exist_ok=True)
+            tsv = ia["outpath"] + "dcr_" + os.path.basename(p1).split(".")[0] + "_beta.tsv"
+            times, digests, device_ctx = {"device": [], "host": []}, {}, None
+            for rep in range(2):
+                for mode in ("device", "host"):
+                    translate._dist = device_ctx if mode == "device" else False
+                    t0 = time.perf_counter()
+                    pipeline._run(dict(ia), frame=False)
+                    times[mode].append(round(time.perf_counter() - t0, 2))
+                    if mode == "device":
+                        device_ctx = translate._dist
+                    digests[mode] = hashlib.sha256(open(tsv, "rb").read()).hexdigest()
+            print(json.dumps({"reads": n, "oligo": args.oligo, "cli_pipeline_s_translate_device": times["device"],
+                              "cli_pipeline_s_translate_host": times["host"], "same_tsv": digests["device"] == digests["host"]}))
+            return
         if args.profile:
             import cProfile, pstats
             pr = cProfile.Profile()
