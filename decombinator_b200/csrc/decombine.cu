@@ -144,7 +144,9 @@ static constexpr int kExactThreads = 512;   // upper bounds; long reads launch n
 #endif
 static constexpr int kGeneralThreads = DCB_GENERAL_THREADS;   // one wide block per SM: the 72 KB of tables are staged once, 24 warps hide the latency
 static constexpr int kMaxChunks = 256;             // queue counters per context
-static constexpr size_t kZeroBlockBytes = sizeof(uint32_t) * 2 * kMaxChunks + sizeof(unsigned long long) * DCB_NCOUNTERS;   // two queue counters per chunk
+// One counter set: two queue counters per chunk, then the reference counters.  A context has two sets (see dcb_run_resident).
+static constexpr size_t kCounterSetWords = 2 * kMaxChunks + 2 * DCB_NCOUNTERS;
+static constexpr size_t kZeroBlockBytes = 2 * kCounterSetWords * sizeof(uint32_t);
 static constexpr uint32_t kChunkReads = 1u << 20;  // reads per chunk of the pipelined host-to-host path
 
 // Shared-memory carve-up common to the kernels: [table 0..3][per-thread columns][counters][mbarrier]
@@ -190,6 +192,33 @@ __device__ __forceinline__ uint32_t exc_first_entry(const BatchDev& b, uint32_t 
     return e;
 }
 
+// Programmatic dependent launch (griddepcontrol, sm_90+).  A resident step launches its kernels with the programmatic
+// stream serialization attribute, so each one is scheduled while its predecessor finishes: before pdl_wait() a kernel
+// touches nothing an earlier kernel writes (shared-memory layout, its own column rows, the constant tag tables); after it,
+// everything the earlier kernels wrote is complete and visible.  EVERY block waits before it exits -- an early exit
+// included -- so a kernel never completes ahead of its predecessor, and a wait on the step's last kernel covers all of
+// them.  Both instructions are no-ops in a kernel launched without the attribute (the chunked paths).
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+// the block's tiles are done: the next kernel of the stream may be scheduled (once every block has said so or exited)
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// Device-side timing of one launch (dcb_timing_*): the earliest block start (stored complemented, so that a zeroed entry
+// takes it with atomicMax) and the latest block end, in %globaltimer nanoseconds.  Null: the launch is not timed.
+struct TierStamp { unsigned long long nstart, end; };
+__device__ __forceinline__ unsigned long long global_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+__device__ __forceinline__ void stamp_start(TierStamp* ts) {
+    if (ts && threadIdx.x == 0) atomicMax(&ts->nstart, ~global_ns());
+}
+__device__ __forceinline__ void stamp_end(TierStamp* ts) {   // block-uniform: called by every thread of the block
+    if (!ts) return;
+    __syncthreads();
+    if (threadIdx.x == 0) atomicMax(&ts->end, global_ns());
+}
+
 // Append the reads of this warp that must go to the general kernel: one atomic per warp.
 __device__ __forceinline__ void defer_reads(bool defer, uint32_t ri, uint32_t* queue, uint32_t* queue_count) {
     const unsigned m = __ballot_sync(0xFFFFFFFFu, defer);
@@ -209,12 +238,14 @@ __device__ __forceinline__ void defer_reads(bool defer, uint32_t ri, uint32_t* q
 __global__ void __launch_bounds__(kExactThreads)
 dcb_exact_kernel(BatchDev b, Tables4 tb, DcrParams prm, int both_frames, dcb_result* __restrict__ results,
                  unsigned long long* __restrict__ counters, uint32_t* __restrict__ queue,
-                 uint32_t* __restrict__ queue_count) {
+                 uint32_t* __restrict__ queue_count, TierStamp* ts) {
+    stamp_start(ts);
     extern __shared__ __align__(16) uint32_t smem[];
     const int T = blockDim.x;
     SmemLayout L = carve(smem, tb, (size_t)b.slot_words * T);
     uint32_t* s_rd = L.cols;  // [slot_words][T]
     stage_tables(L, tb);
+    pdl_wait();
 
     const int tid = threadIdx.x;
     const uint32_t n_tiles = (b.n_reads + T - 1) / T;
@@ -247,7 +278,9 @@ dcb_exact_kernel(BatchDev b, Tables4 tb, DcrParams prm, int both_frames, dcb_res
         defer_reads(live && action == FAST_DEFER, ri, queue, queue_count);
         if (live && action == FAST_DONE) store_result(results + ri, out);
     }
+    pdl_launch_dependents();
     flush_counters(L.cnt, counters);
+    stamp_end(ts);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -345,7 +378,8 @@ template <int NW, int QV, int SV, int WBV, int QJ, int SJ, int WBJ, bool UNION>
 __global__ void __launch_bounds__(1024, 1)
 dcb_exact_kernel_spec(BatchDev b, Tables4 tb, SpecBlooms bl, DcrParams prm, int both_frames, dcb_result* __restrict__ results,
                       unsigned long long* __restrict__ counters, uint32_t* __restrict__ queue,
-                      uint32_t* __restrict__ queue_count) {
+                      uint32_t* __restrict__ queue_count, TierStamp* ts) {
+    stamp_start(ts);
     static_assert(!UNION || (QV == QJ && SV == SJ && WBV == WBJ), "union scan needs one seed geometry");
     using ScanV = SeedScan<NW, QV, SV, WBV>;
     using ScanJ = SeedScan<NW, QJ, SJ, WBJ>;
@@ -365,6 +399,7 @@ dcb_exact_kernel_spec(BatchDev b, Tables4 tb, SpecBlooms bl, DcrParams prm, int 
     s_rd[tid] = 0u;
     for (int k = 0; k < TRAIL; k++) s_rd[(1 + NW + k) * T + tid] = 0u;
     stage_tables(L, tb);
+    pdl_wait();
 
     const DcbTag* vtags = gene_tags(smem);                       // table 0 starts the dynamic shared memory
     const DcbTag* jtags = gene_tags(smem + tb.words[0]);
@@ -432,7 +467,9 @@ dcb_exact_kernel_spec(BatchDev b, Tables4 tb, SpecBlooms bl, DcrParams prm, int 
                                                            : make_uint4(DCB_HIT_UNKNOWN, DCB_HIT_UNKNOWN, flagged ? exc_first_entry(b, ri) : 0u, 0u);
         }
     }
+    pdl_launch_dependents();
     flush_counters(L.cnt, counters);
+    stamp_end(ts);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -476,7 +513,8 @@ template <int NW, int Q, int S, int T, bool EXC>
 __global__ void __launch_bounds__(T, 1)
 dcb_exact_kernel_flat(BatchDev b, QTables qt, DcrParams prm, int both_frames, dcb_result* __restrict__ results,
                       unsigned long long* __restrict__ counters, uint32_t* __restrict__ queue,
-                      uint32_t* __restrict__ queue_count) {
+                      uint32_t* __restrict__ queue_count, TierStamp* ts) {
+    stamp_start(ts);
     static_assert(S == 8, "seeds start at half-word boundaries");
     constexpr int NPOS = (16 * NW - Q) / S + 1;
     constexpr int NA = NPOS < 32 ? NPOS : 32, NB = NPOS - NA;        // probes in the first / second hit word
@@ -514,6 +552,7 @@ dcb_exact_kernel_flat(BatchDev b, QTables qt, DcrParams prm, int both_frames, dc
     if (tid < DCB_NCOUNTERS) s_cnt[tid] = 0;
     tma_stage_wait(bar);
     __syncthreads();
+    pdl_wait();
 
     const DcbTag* vtags = gene_tags(s_vcore);
     const DcbTag* jtags = gene_tags(s_jcore);
@@ -672,7 +711,9 @@ dcb_exact_kernel_flat(BatchDev b, QTables qt, DcrParams prm, int both_frames, dc
             *reinterpret_cast<uint4*>(results + ri) = hand;
         }
     }
+    pdl_launch_dependents();
     flush_counters(s_cnt, counters);
+    stamp_end(ts);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -705,14 +746,17 @@ template <int NW, int T>
 __global__ void __launch_bounds__(T, 1)
 dcb_halftag_kernel(BatchDev b, Tables4 tb, DcrParams prm, dcb_result* __restrict__ results,
                    unsigned long long* __restrict__ counters, const uint32_t* __restrict__ queue,
-                   const uint32_t* __restrict__ queue_count, uint32_t* __restrict__ queue2, uint32_t* __restrict__ queue2_count) {
+                   const uint32_t* __restrict__ queue_count, uint32_t* __restrict__ queue2, uint32_t* __restrict__ queue2_count,
+                   TierStamp* ts) {
     constexpr int ROWS = NW + 3;                                    // a zero row in front of the read's words, two behind
     constexpr int NPOS = (16 * NW - DCB_HALF_Q) / DCB_HALF_STRIDE + 1;
     constexpr int NM = (NPOS + 31) / 32;                            // probe-hit mask words
     static_assert(NM <= 3 && NPOS <= 255, "three mask words, probe index in 8 bits");
+    stamp_start(ts);
+    pdl_wait();
     const uint32_t n_items = *queue_count;
     const uint32_t n_tiles = (n_items + T - 1) / T;
-    if (blockIdx.x >= n_tiles) return;                              // nothing queued for this block: do not even stage the tables
+    if (blockIdx.x >= n_tiles) { stamp_end(ts); return; }          // nothing queued for this block: do not even stage the tables
     extern __shared__ __align__(16) uint32_t smem[];
     const int tid = threadIdx.x, lane = tid & 31, wbase = tid - lane;
     SmemLayout L = carve(smem, tb, (size_t)(2 * ROWS + DCB_HALF_CAP + 1) * T + (size_t)(T / 32) * (DCB_HALF_WCAP / 2 + 2 * DCB_HALF_WCAP2 + 2));
@@ -951,7 +995,9 @@ dcb_halftag_kernel(BatchDev b, Tables4 tb, DcrParams prm, dcb_result* __restrict
         defer_reads(pass_on, ri, queue2, queue2_count);
         __syncwarp();
     }
+    pdl_launch_dependents();
     flush_counters(L.cnt, counters);
+    stamp_end(ts);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -963,9 +1009,15 @@ dcb_halftag_kernel(BatchDev b, Tables4 tb, DcrParams prm, dcb_result* __restrict
 __global__ void __launch_bounds__(kGeneralThreads, DCB_GENERAL_BLOCKS)
 dcb_general_kernel(BatchDev b, Tables4 tb, DcrParams prm, int both_frames, dcb_result* __restrict__ results,
                    unsigned long long* __restrict__ counters, const uint32_t* __restrict__ queue,
-                   const uint32_t* __restrict__ queue_count) {
+                   const uint32_t* __restrict__ queue_count, uint32_t* __restrict__ zero_next, TierStamp* ts) {
     extern __shared__ __align__(16) uint32_t smem[];
     const int T = blockDim.x;
+    stamp_start(ts);
+    pdl_wait();
+    // the last kernel of a resident step clears the counter set of the NEXT step (dcb_run_resident): every kernel that
+    // used that set -- the previous step's -- has completed by now, and the next step's kernels wait for this one
+    if (zero_next && blockIdx.x == 0)
+        for (int i = threadIdx.x; i < (int)kCounterSetWords; i += T) zero_next[i] = 0u;
     // A short queue is spread thinly: S reads per warp (lanes 0 .. S-1), so that all of it runs in one wave of warps and a
     // warp serialises S divergent paths instead of 32 -- the reads that get here are the odd ones, each on a path of its
     // own, and a tile's latency is its slowest warp's (measured on configs[2]: 9 k reads took 0.16 ms at 32 per warp).
@@ -977,7 +1029,7 @@ dcb_general_kernel(BatchDev b, Tables4 tb, DcrParams prm, int both_frames, dcb_r
     }
     const uint32_t per_tile = (uint32_t)(T >> 5) * S;
     const uint32_t n_tiles = (n_items + per_tile - 1) / per_tile;
-    if (blockIdx.x >= n_tiles) return;   // nothing for this block: do not even stage the tables
+    if (blockIdx.x >= n_tiles) { stamp_end(ts); return; }   // nothing for this block: do not even stage the tables
     const int nw = (int)b.slot_words, nwi = (nw + 1) / 2;
     SmemLayout L = carve(smem, tb, (size_t)(nw + nwi) * T * (both_frames ? 2 : 1) + (size_t)(nwi + DCB_HITS_CAP + 6) * T + 20);
     uint32_t* s_rd = L.cols;                      // [nw][T]
@@ -1059,7 +1111,9 @@ dcb_general_kernel(BatchDev b, Tables4 tb, DcrParams prm, int both_frames, dcb_r
             store_result(results + ri, out);
         }
     }
+    pdl_launch_dependents();
     flush_counters(L.cnt, counters);
+    stamp_end(ts);
 }
 
 #include "pack_device.cuh"
@@ -1140,13 +1194,13 @@ struct dcb_ctx {
     DevBuf words, lens, flags, exc_read, exc_pos, exc_kind, exc_index, results, queue;
     std::vector<uint32_t> h_exc_index;   // host copy of exc_index while its upload is in flight
     uint32_t exc_cap = 0;                // entries of the device-side exception list of the batch being packed on the device
-    uint32_t* d_queue_count = nullptr;
-    unsigned long long* d_counters = nullptr;
+    uint32_t* d_queue_count = nullptr;   // two counter sets of kCounterSetWords (dcb_run_resident alternates them)
+    int set_last = 0, set_next = 0;      // the set the last run used; the (zeroed) set the next resident step uses
     BatchDev batch{};
     bool have_batch = false, ran = false;
     bool timing = false;
-    struct Ev { cudaEvent_t a, b; int slot; };
-    std::vector<Ev> events;
+    TierStamp* d_stamps = nullptr;       // one entry per timed launch since the last collection
+    std::vector<int> stamp_slot;         // the timer slot of each entry in use
     double ms[DCB_NTIMERS] = {0, 0, 0, 0};
     uint64_t launches[DCB_NTIMERS] = {0, 0, 0, 0};
     int exact_grid = 0, general_grid = 0, exact_threads = kExactThreads, general_threads = kGeneralThreads;
@@ -1161,7 +1215,7 @@ struct dcb_ctx {
     bool spec_union = false;
 };
 
-typedef void (*exact_spec_fn)(BatchDev, Tables4, SpecBlooms, DcrParams, int, dcb_result*, unsigned long long*, uint32_t*, uint32_t*);
+typedef void (*exact_spec_fn)(BatchDev, Tables4, SpecBlooms, DcrParams, int, dcb_result*, unsigned long long*, uint32_t*, uint32_t*, TierStamp*);
 
 // Specialisations compiled in: V seeds (q=9, stride 12) -- every shipped V tag set has 20-nt minimum tags --
 // with J either sharing that geometry (20-nt J tags: one union index) or using (q=8, stride 5) (12-nt J tags).
@@ -1183,7 +1237,7 @@ static exact_spec_fn pick_spec(int nw, int qv, int sv, int lminv, int qj, int sj
 }
 // Flat kernel: chains whose V and J tags share one index with 20-nt minimum tags (13-mer seeds at stride 8), read slots
 // up to 20 words (320 nt: two hit words).
-typedef void (*exact_q_fn)(BatchDev, QTables, DcrParams, int, dcb_result*, unsigned long long*, uint32_t*, uint32_t*);
+typedef void (*exact_q_fn)(BatchDev, QTables, DcrParams, int, dcb_result*, unsigned long long*, uint32_t*, uint32_t*, TierStamp*);
 static constexpr int kQThreads = 1024;
 static exact_q_fn pick_q(int nw, int qq, int qs, int lmin, bool exc) {
     if (qq != 13 || qs != 8 || lmin != 20) return nullptr;
@@ -1203,7 +1257,8 @@ static int q_rows(int nw) {   // must match the kernel's ROWS
     return 1 + nw + trail;
 }
 
-typedef void (*halftag_fn)(BatchDev, Tables4, DcrParams, dcb_result*, unsigned long long*, const uint32_t*, const uint32_t*, uint32_t*, uint32_t*);
+typedef void (*halftag_fn)(BatchDev, Tables4, DcrParams, dcb_result*, unsigned long long*, const uint32_t*, const uint32_t*, uint32_t*, uint32_t*,
+                           TierStamp*);
 // block width per slot size: as wide as the read / invalid-base / candidate columns leave room for beside the tables
 static halftag_fn pick_half(int nw, int attempt, int* threads) {
     // widest first; the later attempts are for tag sets whose tables leave less room
@@ -1238,33 +1293,48 @@ static int upload_blob(const std::vector<uint32_t>& v, uint32_t** d, int* words)
     return DCB_OK;
 }
 
-static int timing_begin(dcb_ctx* c, int slot) {
-    if (!c->timing) return DCB_OK;
-    dcb_ctx::Ev ev;
-    ev.slot = slot;
-    CUDA_TRY(cudaEventCreate(&ev.a));
-    CUDA_TRY(cudaEventCreate(&ev.b));
-    CUDA_TRY(cudaEventRecord(ev.a, c->stream));
-    c->events.push_back(ev);
-    return DCB_OK;
-}
-static int timing_end(dcb_ctx* c) {
-    if (!c->timing) return DCB_OK;
-    CUDA_TRY(cudaEventRecord(c->events.back().b, c->stream));
-    return DCB_OK;
-}
+// Per-launch timing without host events between the launches (they would end the programmatic overlap of a resident
+// step): each timed kernel stamps its entry of d_stamps itself (TierStamp); the entries are added up, and zeroed for
+// reuse, when they are collected -- by dcb_timing_get / dcb_timing_reset, or when every entry is in use.
+static constexpr int kStamps = 4096;
 static int timing_collect(dcb_ctx* c) {
-    for (auto& ev : c->events) {
-        CUDA_TRY(cudaEventSynchronize(ev.b));
-        float t = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&t, ev.a, ev.b));
-        c->ms[ev.slot] += t;
-        c->launches[ev.slot] += 1;
-        cudaEventDestroy(ev.a);
-        cudaEventDestroy(ev.b);
+    if (c->stamp_slot.empty()) return DCB_OK;
+    std::vector<TierStamp> h(c->stamp_slot.size());
+    CUDA_TRY(cudaMemcpyAsync(h.data(), c->d_stamps, h.size() * sizeof(TierStamp), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemsetAsync(c->d_stamps, 0, h.size() * sizeof(TierStamp), c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    for (size_t i = 0; i < h.size(); i++) {
+        const unsigned long long t0 = ~h[i].nstart;
+        if (h[i].nstart == 0 || h[i].end < t0) continue;   // not stamped (a launch that failed)
+        c->ms[c->stamp_slot[i]] += (double)(h[i].end - t0) * 1e-6;
+        c->launches[c->stamp_slot[i]] += 1;
     }
-    c->events.clear();
+    c->stamp_slot.clear();
     return DCB_OK;
+}
+// The entry a timed launch of timer `slot` stamps, or null when timing is off.
+static int timing_entry(dcb_ctx* c, int slot, bool timed, TierStamp** ts) {
+    *ts = nullptr;
+    if (!timed || !c->timing) return DCB_OK;
+    if ((int)c->stamp_slot.size() == kStamps) {
+        int rc;
+        if ((rc = timing_collect(c))) return rc;
+    }
+    *ts = c->d_stamps + c->stamp_slot.size();
+    c->stamp_slot.push_back(slot);
+    return DCB_OK;
+}
+
+// A kernel launch; pdl: with the programmatic stream serialization attribute (see pdl_wait).
+template <typename... P, typename... A>
+static cudaError_t launch(bool pdl, void (*fn)(P...), int grid, int threads, size_t smem, cudaStream_t s, A... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)threads); cfg.dynamicSmemBytes = smem; cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, fn, args...);
 }
 
 extern "C" {
@@ -1329,9 +1399,10 @@ dcb_ctx* dcb_ctx_create(int device, const dcb_tagset* v, const dcb_tagset* j, co
         if (dcb_build_half_index(v, j, hb))
             if (upload_blob(hb, &c->d_half, &c->half_words)) return fail(nullptr);
     }
-    // queue counters and reference counters in ONE block: a step clears both with one memset
+    // queue counters and reference counters in ONE block (both counter sets): one memset clears them all
     if (cudaMalloc((void**)&c->d_queue_count, kZeroBlockBytes) != cudaSuccess) return fail("cudaMalloc");
-    c->d_counters = reinterpret_cast<unsigned long long*>(c->d_queue_count + 2 * kMaxChunks);
+    if (cudaMemsetAsync(c->d_queue_count, 0, kZeroBlockBytes, c->own_stream) != cudaSuccess ||
+        cudaStreamSynchronize(c->own_stream) != cudaSuccess) return fail("cudaMemset");
     if (cudaMalloc((void**)&c->d_exc_total, 16) != cudaSuccess) return fail("cudaMalloc");
     for (int i = 0; i < 2; i++)
         if (cudaEventCreateWithFlags(&c->ev_scan[i], cudaEventDisableTiming) != cudaSuccess ||
@@ -1345,14 +1416,14 @@ dcb_ctx* dcb_ctx_create(int device, const dcb_tagset* v, const dcb_tagset* j, co
 void dcb_ctx_destroy(dcb_ctx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
-    timing_collect(c);
     if (c->own_stream) { cudaStreamSynchronize(c->own_stream); cudaStreamDestroy(c->own_stream); }
     if (c->stream2) { cudaStreamSynchronize(c->stream2); cudaStreamDestroy(c->stream2); }
     if (c->ev_ready) cudaEventDestroy(c->ev_ready);
     if (c->ev_done) cudaEventDestroy(c->ev_done);
     cudaFree(c->d_vgen); cudaFree(c->d_jgen); cudaFree(c->d_vcore); cudaFree(c->d_jcore);
     cudaFree(c->d_vidx); cudaFree(c->d_jidx); cudaFree(c->d_uidx); cudaFree(c->d_sfilt); cudaFree(c->d_half);
-    cudaFree(c->d_queue_count);   // d_counters lives in the same block
+    cudaFree(c->d_queue_count);   // the reference counters live in the same block
+    cudaFree(c->d_stamps);
     c->words.release(); c->lens.release(); c->flags.release(); c->exc_read.release(); c->exc_pos.release(); c->exc_index.release();
     c->exc_kind.release(); c->results.release(); c->queue.release(); c->queue2.release();
     for (int i = 0; i < 2; i++) {
@@ -1512,22 +1583,34 @@ static int copy_side_arrays(dcb_ctx* c, const dcb_packed* P, cudaStream_t s) {
     return DCB_OK;
 }
 
-// Both kernels over reads [first, first + count) of the resident batch, on stream s.  slot: which queue counter.
-static int launch_range(dcb_ctx* c, cudaStream_t s, uint32_t first, uint32_t count, int slot, bool timed) {
+static uint32_t* counter_set(dcb_ctx* c, int set) { return c->d_queue_count + (size_t)set * kCounterSetWords; }
+static unsigned long long* ref_counters(dcb_ctx* c, int set) {
+    return reinterpret_cast<unsigned long long*>(counter_set(c, set) + 2 * kMaxChunks);
+}
+
+// The kernels over reads [first, first + count) of the resident batch, on stream s.  set, slot: which counter set and
+// which queue counters in it.  zero_next: the counter set the general kernel clears for the next step (or null).  pdl:
+// every launch with the programmatic stream serialization attribute (dcb_run_resident).
+static int launch_range(dcb_ctx* c, cudaStream_t s, uint32_t first, uint32_t count, int set, int slot, uint32_t* zero_next,
+                        bool timed, bool pdl) {
     if (count == 0) return DCB_OK;
     BatchDev b = c->batch;
     b.first = first; b.n_reads = count;
-    uint32_t* qcount = c->d_queue_count + slot;
+    uint32_t* qcount = counter_set(c, set) + slot;
+    unsigned long long* counters = ref_counters(c, set);
     uint32_t* queue = (uint32_t*)c->queue.p + first;
+    dcb_result* results = (dcb_result*)c->results.p;
     DcrParams prm;
     prm.allow_ns = c->params.allow_ns; prm.lenthreshold = c->params.lenthreshold;
     const uint32_t tiles_e = (count + c->exact_threads - 1) / c->exact_threads;
     const uint32_t tiles_g = (count + c->general_threads - 1) / c->general_threads;
     const int grid_e = (int)std::max<uint32_t>(1, std::min<uint32_t>(tiles_e, (uint32_t)c->exact_grid));
     const int grid_g = (int)std::max<uint32_t>(1, std::min<uint32_t>(tiles_g, (uint32_t)c->general_grid));
+    const int both = c->params.both_frames;
+    TierStamp* ts;
     int rc;
     if (c->params.force_general != 1) {
-        if (timed && (rc = timing_begin(c, 0))) return rc;
+        if ((rc = timing_entry(c, 0, timed, &ts))) return rc;
         Tables4 te;
         te.g[0] = c->d_vcore; te.words[0] = c->vcore_words;
         te.g[1] = c->d_jcore; te.words[1] = c->jcore_words;
@@ -1538,51 +1621,51 @@ static int launch_range(dcb_ctx* c, cudaStream_t s, uint32_t first, uint32_t cou
             qt.vcore = c->d_vcore; qt.jcore = c->d_jcore; qt.head = c->d_uidx; qt.qtab = c->d_uidx + c->uqtab_off;
             qt.bfilter = c->d_uidx + c->ubfilter_off;
             qt.vcore_words = c->vcore_words; qt.jcore_words = c->jcore_words; qt.head_words = c->uhead; qt.qtab_words = c->uqtab_words;
-            ((exact_q_fn)c->q_fn)<<<grid_e, c->exact_threads, c->exact_smem, s>>>(
-                b, qt, prm, c->params.both_frames, (dcb_result*)c->results.p, c->d_counters, queue, qcount);
+            CUDA_TRY(launch(pdl, (exact_q_fn)c->q_fn, grid_e, c->exact_threads, c->exact_smem, s, b, qt, prm, both, results, counters,
+                            queue, qcount, ts));
         } else if (c->spec_fn) {
             SpecBlooms sb;
             if (c->spec_union) { te.words[2] = c->uhead; sb.v = c->d_uidx + c->ubloom; sb.j = nullptr; }
             else { te.words[2] = c->vhead; te.words[3] = c->jhead; sb.v = c->d_vidx + c->vbloom; sb.j = c->d_jidx + c->jbloom; }
-            ((exact_spec_fn)c->spec_fn)<<<grid_e, c->exact_threads, c->exact_smem, s>>>(
-                b, te, sb, prm, c->params.both_frames, (dcb_result*)c->results.p, c->d_counters, queue, qcount);
+            CUDA_TRY(launch(pdl, (exact_spec_fn)c->spec_fn, grid_e, c->exact_threads, c->exact_smem, s, b, te, sb, prm, both, results,
+                            counters, queue, qcount, ts));
         } else {
-            dcb_exact_kernel<<<grid_e, c->exact_threads, c->exact_smem, s>>>(
-                b, te, prm, c->params.both_frames, (dcb_result*)c->results.p, c->d_counters, queue, qcount);
+            CUDA_TRY(launch(pdl, dcb_exact_kernel, grid_e, c->exact_threads, c->exact_smem, s, b, te, prm, both, results, counters,
+                            queue, qcount, ts));
         }
-        CUDA_TRY(cudaGetLastError());
-        if (timed && (rc = timing_end(c))) return rc;
     }
     Tables4 tg;
     tg.g[3] = nullptr; tg.words[3] = 0;
     if (c->half_fn) {   // the queued reads through the half-tag kernel; what it passes on is the general kernel's queue
-        if (timed && (rc = timing_begin(c, 2))) return rc;
-        uint32_t* qcount2 = c->d_queue_count + kMaxChunks + slot;
+        if ((rc = timing_entry(c, 2, timed, &ts))) return rc;
+        uint32_t* qcount2 = counter_set(c, set) + kMaxChunks + slot;
         uint32_t* queue2 = (uint32_t*)c->queue2.p + first;
         tg.g[0] = c->d_vcore; tg.words[0] = c->vcore_words; tg.g[1] = c->d_jcore; tg.words[1] = c->jcore_words;
         tg.g[2] = c->d_half; tg.words[2] = c->half_words;
         const uint32_t tiles_h = (count + c->half_threads - 1) / c->half_threads;
         const int grid_h = (int)std::max<uint32_t>(1, std::min<uint32_t>(tiles_h, (uint32_t)c->half_grid));
-        ((halftag_fn)c->half_fn)<<<grid_h, c->half_threads, c->half_smem, s>>>(
-            b, tg, prm, (dcb_result*)c->results.p, c->d_counters, queue, qcount, queue2, qcount2);
-        CUDA_TRY(cudaGetLastError());
-        if (timed && (rc = timing_end(c))) return rc;
+        CUDA_TRY(launch(pdl, (halftag_fn)c->half_fn, grid_h, c->half_threads, c->half_smem, s, b, tg, prm, results, counters,
+                        (const uint32_t*)queue, (const uint32_t*)qcount, queue2, qcount2, ts));
         queue = queue2; qcount = qcount2;
     }
-    if (timed && (rc = timing_begin(c, 1))) return rc;
+    if ((rc = timing_entry(c, 1, timed, &ts))) return rc;
     tg.g[0] = c->d_vgen; tg.words[0] = c->vgen_words; tg.g[1] = c->d_jgen; tg.words[1] = c->jgen_words;
     tg.g[2] = c->d_sfilt; tg.words[2] = c->sfilt_words;
-    dcb_general_kernel<<<grid_g, c->general_threads, c->general_smem, s>>>(
-        b, tg, prm, c->params.both_frames, (dcb_result*)c->results.p, c->d_counters,
-        c->params.force_general == 1 ? nullptr : (const uint32_t*)queue, qcount);
-    CUDA_TRY(cudaGetLastError());
-    if (timed && (rc = timing_end(c))) return rc;
+    CUDA_TRY(launch(pdl, dcb_general_kernel, grid_g, c->general_threads, c->general_smem, s, b, tg, prm, both, results, counters,
+                    c->params.force_general == 1 ? nullptr : (const uint32_t*)queue, (const uint32_t*)qcount, zero_next, ts));
+    return DCB_OK;
+}
+
+// Clear both counter sets on stream s: the chunked paths count in set 0, the next resident step in set 1.
+static int reset_counter_sets(dcb_ctx* c, cudaStream_t s) {
+    CUDA_TRY(cudaMemsetAsync(c->d_queue_count, 0, kZeroBlockBytes, s));
+    c->set_last = 0; c->set_next = 1;
     return DCB_OK;
 }
 
 static int read_counters(dcb_ctx* c, cudaStream_t s, uint64_t* counters) {
     unsigned long long h[DCB_NCOUNTERS];
-    CUDA_TRY(cudaMemcpyAsync(h, c->d_counters, sizeof(h), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(h, ref_counters(c, c->set_last), sizeof(h), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
     if (counters) for (int i = 0; i < DCB_NCOUNTERS; i++) counters[i] += h[i];
     return DCB_OK;
@@ -1597,7 +1680,7 @@ static uint32_t chunk_reads(uint32_t base, uint64_t n) {
 // The chunk's kernels (chunk_no: its queue counters) and, when out is given, its result records back to the host.
 static int run_chunk(dcb_ctx* c, cudaStream_t s, uint32_t first, uint32_t count, int chunk_no, dcb_result* out) {
     int rc;
-    if ((rc = launch_range(c, s, first, count, chunk_no, false))) return rc;
+    if ((rc = launch_range(c, s, first, count, 0, chunk_no, nullptr, false, false))) return rc;
     if (out)
         CUDA_TRY(cudaMemcpyAsync(out + first, (dcb_result*)c->results.p + first, (size_t)count * sizeof(dcb_result),
                                  cudaMemcpyDeviceToHost, s));
@@ -1631,13 +1714,30 @@ int dcb_upload(dcb_ctx* c, const dcb_packed* P) {
     return DCB_OK;
 }
 
+// A resident step is its kernels alone, chained by programmatic dependent launch (pdl_wait): step k + 1's exact kernel
+// stages its tables while step k's last kernels finish, and a follow-up kernel with nothing queued costs an early exit of
+// blocks already resident, not a launch behind a drained grid.  A memset in the stream would end that overlap, so the
+// steps alternate between the two counter sets: a step counts in the set the step before it left zeroed, and its general
+// kernel zeroes the other one for the step after it.  DCB_PDL=0: plain launches behind a memset of both sets (A/B runs).
 int dcb_run_resident(dcb_ctx* c) {
     if (!c || !c->have_batch) { dcb_set_error("dcb_run_resident: no batch uploaded"); return DCB_EINVAL; }
+    const char* e = std::getenv("DCB_PDL");
+    if (e && std::strcmp(e, "0") && std::strcmp(e, "1")) {
+        dcb_set_error("DCB_PDL=%s: accepted values are 1 (the default: the kernels of a step chained by programmatic dependent "
+                      "launch) and 0 (plain launches behind a memset of the counters)", e);
+        return DCB_EINVAL;
+    }
+    const bool pdl = !e || e[0] == '1';
     CUDA_TRY(cudaSetDevice(c->device));
     cudaStream_t s = c->stream;
-    CUDA_TRY(cudaMemsetAsync(c->d_queue_count, 0, kZeroBlockBytes, s));
     int rc;
-    if ((rc = launch_range(c, s, 0, c->batch.n_reads, 0, true))) return rc;
+    if (!pdl && (rc = reset_counter_sets(c, s))) return rc;
+    const int set = c->set_next;
+    if ((rc = launch_range(c, s, 0, c->batch.n_reads, set, 0, pdl ? counter_set(c, 1 - set) : nullptr, true, pdl))) return rc;
+    // An empty batch launches nothing, so no general kernel zeroes the other set: the step reports the (zeroed) set it
+    // would have counted in, and the next step counts there again.
+    c->set_last = set;
+    if (c->batch.n_reads) c->set_next = 1 - set;
     c->ran = true;
     return DCB_OK;
 }
@@ -1662,7 +1762,7 @@ int dcb_decombine_batch(dcb_ctx* c, const dcb_packed* P, dcb_result* out, uint64
     const uint32_t n = (uint32_t)P->n_reads;
     const size_t sw = P->slot_words;
     cudaStream_t st[2] = {c->stream, c->stream2};
-    CUDA_TRY(cudaMemsetAsync(c->d_queue_count, 0, kZeroBlockBytes, st[0]));
+    if ((rc = reset_counter_sets(c, st[0]))) return rc;
     if ((rc = copy_side_arrays(c, P, st[0]))) return rc;
     if ((rc = fork_streams(c, st))) return rc;
     const uint32_t chunk = chunk_reads(kChunkReads, n);
@@ -2038,7 +2138,7 @@ int dcb_decombine_ascii(dcb_ctx* c, const char* ascii, const uint64_t* off, cons
     if ((rc = ascii_begin(c, ascii, off, len, n, uniform_len, &exc_cap))) return rc;
     const uint32_t* lens = uniform_len ? nullptr : len;
     cudaStream_t st[2] = {c->stream, c->stream2};
-    CUDA_TRY(cudaMemsetAsync(c->d_queue_count, 0, kZeroBlockBytes, st[0]));
+    if ((rc = reset_counter_sets(c, st[0]))) return rc;
     if ((rc = fork_streams(c, st))) return rc;
     // text in pageable memory (a memory-mapped file): smaller chunks through page-locked staging buffers
     bool staged = false;
@@ -2147,7 +2247,17 @@ void* dcb_pinned_alloc(size_t bytes) {
 }
 void dcb_pinned_free(void* p) { if (p) cudaFreeHost(p); }
 
-int dcb_timing_enable(dcb_ctx* c, int on) { if (!c) return DCB_EINVAL; c->timing = on != 0; return DCB_OK; }
+int dcb_timing_enable(dcb_ctx* c, int on) {
+    if (!c) return DCB_EINVAL;
+    if (on && !c->d_stamps) {   // zeroed before the first timed launch: the stamps are taken with atomicMax
+        CUDA_TRY(cudaSetDevice(c->device));
+        CUDA_TRY(cudaMalloc((void**)&c->d_stamps, kStamps * sizeof(TierStamp)));
+        CUDA_TRY(cudaMemset(c->d_stamps, 0, kStamps * sizeof(TierStamp)));
+        CUDA_TRY(cudaDeviceSynchronize());
+    }
+    c->timing = on != 0;
+    return DCB_OK;
+}
 int dcb_timing_reset(dcb_ctx* c) {
     if (!c) return DCB_EINVAL;
     int rc = timing_collect(c);
@@ -2167,7 +2277,7 @@ const char* dcb_exact_kernel_name(const dcb_ctx* c) {
 static int sum_queue_counts(dcb_ctx* c, int which, uint64_t* total) {
     uint32_t q[kMaxChunks];
     CUDA_TRY(cudaStreamSynchronize(c->stream));
-    CUDA_TRY(cudaMemcpy(q, c->d_queue_count + which * kMaxChunks, sizeof(q), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(q, counter_set(c, c->set_last) + which * kMaxChunks, sizeof(q), cudaMemcpyDeviceToHost));
     *total = 0;
     for (int i = 0; i < kMaxChunks; i++) *total += q[i];
     return DCB_OK;

@@ -277,14 +277,19 @@ void dcb_pinned_free(void*);
 
 /* Same work with the batch resident in HBM (bench `value`, multi-step pipelines):
  *   dcb_upload          : host packed batch -> ctx-owned device buffers (synchronous)
- *   dcb_run_resident    : launch the kernels on the resident batch; asynchronous on the ctx stream
+ *   dcb_run_resident    : launch the kernels on the resident batch; asynchronous on the ctx stream.  The kernels of
+ *                         consecutive steps are chained by programmatic dependent launch; the environment variable
+ *                         DCB_PDL = 0 launches them plainly behind a memset of the counters, a value other than 0 or 1
+ *                         fails the call with DCB_EINVAL
  *   dcb_download        : wait, copy results + ADD counter deltas of the last run
  */
 int dcb_upload(dcb_ctx*, const dcb_packed* reads);
 int dcb_run_resident(dcb_ctx*);
 int dcb_download(dcb_ctx*, dcb_result* out, uint64_t* counters);
 
-/* Per-kernel device time (CUDA events on the launching stream), accumulated since the last reset.
+/* Per-kernel device time of the resident steps, accumulated since the last reset, and the number of launches timed.
+ * A launch's time runs from the start of its first block to the end of its last block (%globaltimer, stamped by the
+ * kernels themselves: no host event sits between the launches of a step).
  * slot 0: exact-tag matching kernel, slot 1: general kernel, slot 2: half-tag kernel. */
 #define DCB_NTIMERS 4
 int dcb_timing_reset(dcb_ctx*);
