@@ -153,6 +153,7 @@ def lib():
     L.dcb_lev_leq.argtypes = [vp, vp, vp, vp, u32, vp, vp, u64, ctypes.c_double, vp]
     L.dcb_lev_leq_bytes.argtypes = [vp, vp, vp, vp, u32, vp, vp, u64, ctypes.c_double, vp]
     L.dcb_barcodes.argtypes = [vp, vp, vp, vp, vp, vp, vp, u64, ctypes.POINTER(CBcParams), vp, vp, vp]
+    L.dcb_barcodes_fuzzy.argtypes = [vp, vp, vp, vp, vp, vp, vp, u64, ctypes.POINTER(CBcParams), i32, vp, vp, vp, vp]
     L.dcb_dist_last_ms.argtypes = [vp, ctypes.POINTER(ctypes.c_double)]
     L.dcb_dist_last_method.argtypes = [vp]
     L.dcb_dist_last_method.restype = ctypes.c_char_p
@@ -983,17 +984,20 @@ class Dist:
                                  a.ctypes.data, b.ctypes.data, len(a), float(frac), out.ctypes.data), "dcb_lev_leq")
         return out.astype(bool)
 
-    def barcodes(self, bcs, quals, oligo, allow_ns, min_q, max_below, avg_q):
+    def barcodes(self, bcs, quals, oligo, allow_ns, min_q, max_below, avg_q, fuzzy=False):
         """dcb_barcodes over lists of barcode-region strings and their quality strings.
-        -> (status uint8, n1len uint8, code uint64) arrays; status BC_HOST rows are for the reference's fuzzy spacer search."""
+        -> (status uint8, n1len uint8, code uint64) arrays; status BC_HOST rows are for the reference's fuzzy spacer search.
+        fuzzy: dcb_barcodes_fuzzy, the fuzzy searches on the device too; -> (status, n1len, code, match uint8)."""
         n = len(bcs)
         if n == 0:
-            return np.zeros(0, dtype=np.uint8), np.zeros(0, dtype=np.uint8), np.zeros(0, dtype=np.uint64)
+            out = np.zeros(0, dtype=np.uint8), np.zeros(0, dtype=np.uint8), np.zeros(0, dtype=np.uint64)
+            return out + (np.zeros(0, dtype=np.uint8),) if fuzzy else out
         try:
             bbuf = np.frombuffer("".join(bcs).encode("ascii") + b"\0", dtype=np.uint8)
             qbuf = np.frombuffer("".join(quals).encode("ascii") + b"\0", dtype=np.uint8)
         except UnicodeEncodeError:                       # non-ASCII text: every row takes the host path
-            return np.full(n, BC_HOST, dtype=np.uint8), np.zeros(n, dtype=np.uint8), np.zeros(n, dtype=np.uint64)
+            out = np.full(n, BC_HOST, dtype=np.uint8), np.zeros(n, dtype=np.uint8), np.zeros(n, dtype=np.uint64)
+            return out + (np.zeros(n, dtype=np.uint8),) if fuzzy else out
         bl = np.fromiter((len(x) for x in bcs), dtype=np.uint32, count=n)
         ql = np.fromiter((len(x) for x in quals), dtype=np.uint32, count=n)
         bo = np.zeros(n, dtype=np.uint64)
@@ -1001,17 +1005,24 @@ class Dist:
         if n > 1:
             np.cumsum(bl[:-1], dtype=np.uint64, out=bo[1:])
             np.cumsum(ql[:-1], dtype=np.uint64, out=qo[1:])
-        return self.barcodes_arrays(bbuf, bo, bl, qbuf, qo, ql, oligo, allow_ns, min_q, max_below, avg_q)
+        return self.barcodes_arrays(bbuf, bo, bl, qbuf, qo, ql, oligo, allow_ns, min_q, max_below, avg_q, fuzzy)
 
-    def barcodes_arrays(self, bbuf, bo, bl, qbuf, qo, ql, oligo, allow_ns, min_q, max_below, avg_q):
-        """dcb_barcodes over (offset, length) columns into two uint8 text buffers."""
+    def barcodes_arrays(self, bbuf, bo, bl, qbuf, qo, ql, oligo, allow_ns, min_q, max_below, avg_q, fuzzy=False):
+        """dcb_barcodes over (offset, length) columns into two uint8 text buffers; fuzzy: dcb_barcodes_fuzzy with its
+        switch on, and the match array as a fourth result."""
         n = len(bo)
         status, n1, code = np.full(n, BC_HOST, dtype=np.uint8), np.zeros(n, dtype=np.uint8), np.zeros(n, dtype=np.uint64)
+        match = np.zeros(n, dtype=np.uint8) if fuzzy else None
         if n == 0:
-            return status, n1, code
+            return (status, n1, code, match) if fuzzy else (status, n1, code)
         bo, qo = np.ascontiguousarray(bo, dtype=np.uint64), np.ascontiguousarray(qo, dtype=np.uint64)
         bl, ql = np.ascontiguousarray(bl, dtype=np.uint32), np.ascontiguousarray(ql, dtype=np.uint32)
         prm = CBcParams(int(oligo), int(bool(allow_ns)), int(min_q), int(max_below), float(avg_q))
+        if fuzzy:
+            _check(lib().dcb_barcodes_fuzzy(self._h, bbuf.ctypes.data, bo.ctypes.data, bl.ctypes.data, qbuf.ctypes.data, qo.ctypes.data,
+                                            ql.ctypes.data, n, ctypes.byref(prm), 1, status.ctypes.data, n1.ctypes.data, code.ctypes.data,
+                                            match.ctypes.data), "dcb_barcodes_fuzzy")
+            return status, n1, code, match
         _check(lib().dcb_barcodes(self._h, bbuf.ctypes.data, bo.ctypes.data, bl.ctypes.data, qbuf.ctypes.data, qo.ctypes.data,
                                   ql.ctypes.data, n, ctypes.byref(prm), status.ctypes.data, n1.ctypes.data, code.ctypes.data), "dcb_barcodes")
         return status, n1, code

@@ -364,16 +364,27 @@ class _BarcodeMachine:
 _BC_SYMBOLS = np.frombuffer(b"ACGTNSL?", dtype=np.uint8)
 
 
+def _fuzzy_on_device(d):
+    """DCB_BC_FUZZY=0: the device leaves rows whose spacers are not found exactly to the host's regex path (A/B runs).
+    A context that is not a _lib.Dist (the CPU tests install the oracle's, which hands every row back) takes the
+    exact-search signature."""
+    return os.environ.get("DCB_BC_FUZZY", "1") != "0" and isinstance(d, _lib.Dist)
+
+
 def _device_barcodes(rows, inputargs, qp):
-    """dcb_barcodes over the barcode regions of all rows at once: -> (status, n1len, barcode strings) or None when this
-    oligo / option has no device path.  Rows whose spacers are not found exactly come back with status BC_HOST."""
+    """dcb_barcodes_fuzzy over the barcode regions of all rows at once: -> (status, barcode strings) or None when this
+    oligo / option has no device path.  Rows with odd symbols, a ragged quality string or an overlong region come back with
+    status BC_HOST (with DCB_BC_FUZZY=0 also rows whose spacers are not found exactly)."""
     name = inputargs["oligo"].lower()
     if name not in _lib.OLIGOS_ON_DEVICE or inputargs["sampling_analysis"] or not rows or "allowNs" not in inputargs:
         return None      # (without the allowNs key the reference fails on the first barcode that holds an N: host path)
-    status, n1, code = _gpu().barcodes([r[8] for r in rows], [r[9] for r in rows], _lib.OLIGOS_ON_DEVICE[name],
-                                       inputargs["allowNs"] != False, qp[0], qp[1], qp[2])  # noqa: E712
+    d = _gpu()
+    fuzzy = _fuzzy_on_device(d)
+    out = d.barcodes([r[8] for r in rows], [r[9] for r in rows], _lib.OLIGOS_ON_DEVICE[name],
+                     inputargs["allowNs"] != False, qp[0], qp[1], qp[2], *((True,) if fuzzy else ()))  # noqa: E712
+    status, n1, code = out[:3]
     text = _decode_barcodes(code, _lib.BC_LENGTH[name])      # BC_LENGTH[name] characters per row, back to back
-    _count_device_barcodes(status, n1, name)
+    _count_device_barcodes(status, n1, name, out[3] if fuzzy else None)
     return status, text
 
 
@@ -383,10 +394,11 @@ def _decode_barcodes(code, width):
     return _BC_SYMBOLS[sym.astype(np.intp)].tobytes().decode("ascii")
 
 
-def _count_device_barcodes(status, n1, name):
-    """The reference's counters for the rows decided on the device (collapse.py:241-278, 388-422, 546-553).  The
-    fixed-barcode designs (NEBIO, TAKARA) have no N1: every placed row counts as getbarcode_pass_other, none as a short
-    or long barcode."""
+def _count_device_barcodes(status, n1, name, match=None):
+    """The reference's counters for the rows decided on the device (collapse.py:241-278, 388-422, 546-553).  match (None:
+    all 0) says which placed rows took a fuzzy spacer text: getbarcode_pass_regexmatch instead of _exactmatch, and
+    logFuzzyMatching's classes by N1 length.  The fixed-barcode designs (NEBIO, TAKARA) have no N1: the reference passes
+    their barcode length for it, so every placed row counts as N1 of the right length, none as a short or long barcode."""
     st = np.bincount(status, minlength=256)
     for key, k in (("getbarcode_fail_N", st[_lib.BC_FAIL_N]), ("getbarcode_fail_nospacerfound", st[_lib.BC_FAIL_NOSPACER]),
                    ("getbarcode_fail_not2spacersfound", st[_lib.BC_FAIL_NOT2]), ("getbarcode_fail_n1tooshort", st[_lib.BC_FAIL_N1SHORT]),
@@ -395,12 +407,16 @@ def _count_device_barcodes(status, n1, name):
                    ("readdata_fail_low_barcode_quality", st[_lib.BC_FAIL_QUALITY])):
         if k:
             counts[key] += int(k)
-    placed = (status == _lib.BC_OK) | (status == _lib.BC_FAIL_QUALITY)         # spacers found exactly, N1 / N2 in range
+    placed = (status == _lib.BC_OK) | (status == _lib.BC_FAIL_QUALITY)         # spacers found, N1 / N2 in range
+    fuzzy = placed & (match != 0) if match is not None else np.zeros_like(placed)
+    exact = placed & ~fuzzy
     if name in _lib.BC_FIXED:
-        other, short, long_ = placed, np.zeros_like(placed), np.zeros_like(placed)
+        right, short, long_ = placed, np.zeros_like(placed), np.zeros_like(placed)
     else:
-        other, short, long_ = placed & (n1 == 6), placed & (n1 < 6), placed & (n1 > 6)
-    for key, k in (("getbarcode_pass_exactmatch", placed.sum()), ("getbarcode_pass_other", other.sum()),
+        right, short, long_ = placed & (n1 == 6), placed & (n1 < 6), placed & (n1 > 6)
+    for key, k in (("getbarcode_pass_exactmatch", exact.sum()), ("getbarcode_pass_regexmatch", fuzzy.sum()),
+                   ("getbarcode_pass_fuzzymatch_rightlen", (fuzzy & right).sum()), ("getbarcode_pass_fuzzymatch_short", (fuzzy & short).sum()),
+                   ("getbarcode_pass_fuzzymatch_long", (fuzzy & long_).sum()), ("getbarcode_pass_other", (exact & right).sum()),
                    ("readdata_short_barcode", short.sum()), ("readdata_long_barcode", long_.sum())):
         if k:
             counts[key] += int(k)
@@ -460,12 +476,15 @@ def _filter_columns(data, inputargs, barcode_quality_parameters, first_index=0):
     name = inputargs["oligo"].lower()
     if name not in _lib.OLIGOS_ON_DEVICE or inputargs["sampling_analysis"] or "allowNs" not in inputargs or len(data) == 0:
         return None
-    status, n1, code = _gpu().barcodes_arrays(*data.barcode_columns(), _lib.OLIGOS_ON_DEVICE[name], inputargs["allowNs"] != False,  # noqa: E712
-                                              *barcode_quality_parameters)
-    _count_device_barcodes(status, n1, name)
+    d = _gpu()
+    fuzzy = _fuzzy_on_device(d)
+    out = d.barcodes_arrays(*data.barcode_columns(), _lib.OLIGOS_ON_DEVICE[name], inputargs["allowNs"] != False,  # noqa: E712
+                            *barcode_quality_parameters, *((True,) if fuzzy else ()))
+    status, n1, code = out[:3]
+    _count_device_barcodes(status, n1, name, out[3] if fuzzy else None)
     ok, host = status == _lib.BC_OK, status == _lib.BC_HOST
     # rows whose barcode the kernel assembled: no Python row at all, the three strings collapse files them under come from
-    # dcb_format_collapse_rows; rows it hands back (fuzzy spacer search) become Python rows as before
+    # dcb_format_collapse_rows; rows it hands back (odd symbols, ragged quality strings) become Python rows as before
     seqs, dcrs, etcs = data.collapse_lines(ok)
     width = _lib.BC_LENGTH[name]
     text = _decode_barcodes(code[ok], width)
@@ -477,9 +496,9 @@ def _filter_columns(data, inputargs, barcode_quality_parameters, first_index=0):
 def _filter_rows(data, inputargs, barcode_quality_parameters, dont_count, from_file, first_index=0):
     """The per-row part of read_in_data (collapse.py:523-593): barcode location, quality and length filters.
 
-    The barcode of every row is located, assembled and quality-checked by ONE kernel launch (dcb_barcodes: exact spacer
-    search); only the rows it hands back -- spacers not found exactly, so the reference's fuzzy regular expressions
-    decide -- go through get_barcode_positions / set_barcode / check_umi_quality on the host.
+    The barcode of every row is located, assembled and quality-checked by ONE kernel launch (dcb_barcodes_fuzzy: the exact
+    spacer search and the reference's fuzzy ones); only the rows it hands back -- odd symbols, ragged quality strings,
+    regions over 250 bases -- go through get_barcode_positions / set_barcode / check_umi_quality on the host.
 
     -> ([(global row index, barcode, seq, dcretc), ...] for the rows that survive, Counter of str(dcr), rows seen).
     Rows are independent here, so a multi-GPU run calls this on each rank's shard (parallel.py)."""

@@ -19,6 +19,7 @@
 //     front of the verifier.
 // The output of both is the device radix sort of the 64-bit (row << 32 | col) keys.
 #include "dcb_internal.h"
+#include "barcode_core.cuh"
 #include "lev_core.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
@@ -288,93 +289,21 @@ dcb_lev_leq_kernel(const uint8_t* __restrict__ sym, const uint64_t* __restrict__
 }
 
 // ---- barcode extraction (SURVEY 8(f) row 3) ------------------------------------------------------------------------
-// One thread per decombined row: the barcode region (R2[:bclength], field 8 of an .n12 row) and its quality string.
-// What collapse.py does per row before any grouping (get_barcode_positions, collapse.py:367-479): an 'N' anywhere rejects
-// the row (unless -N); spacer 1 is searched in its window bc[lo:hi] and must be found exactly once (regex.findall:
-// leftmost, non-overlapping).  Then, per layout of the ligation oligo:
-//   two spacers (M13, I8): window bc[0 : 10 + len(spacer1)]; spacer 2 is searched in bc[len(spacer1):] and must be found
-//     exactly once; N1 lies between the spacers, N2 is the six bases behind spacer 2;
-//   N1, spacer, N2 (I8_single): window bc[0:18]; N1 is bc[0 : spacer position], N2 the six bases behind the spacer;
-//     for both: N1 of <= 3 or >= 9 bases and an N2 that runs past the end reject the row, and set_barcode (:281-326)
-//     makes N1 + N2, a short N1 padded with 'S' (quality '?'), a long one cut to five bases + 'L';
-//   fixed barcode (NEBIO: window bc[18:28], barcode bc[0:17]; TAKARA: window bc[0:19], barcode bc[0:12]): the spacer only
-//     has to be there, its position is not used.
-// check_umi_quality (:340-352): more than `max_below` barcode qualities under `min_q`, or a mean under `avg_q`, rejects the row.
-// Only the EXACT spacer search is done here.  The reference escalates to fuzzy regular expressions ({1s<=2}, then
-// {2i+2d+1s<=2}) when an exact search finds nothing: such rows (a few percent) come back as DCB_BC_HOST and the host
-// runs the reference's own search on them; so do rows with symbols outside ACGTN, a quality string of another length, a
-// region longer than 250, and fixed-barcode regions shorter than the barcode (the reference would cut the barcode short).
-__device__ __forceinline__ int bc_find(const unsigned char* s, int from, int to, const char* pat, int plen) {   // first match in [from, to)
-    for (int p = from; p + plen <= to; p++) {
-        int k = 0;
-        while (k < plen && s[p + k] == (unsigned char)pat[k]) k++;
-        if (k == plen) return p;
-    }
-    return -1;
-}
-__device__ __forceinline__ int bc_count(const unsigned char* s, int from, int to, const char* pat, int plen, int& first) {
-    int n = 0;
-    first = -1;
-    for (int p = bc_find(s, from, to, pat, plen); p >= 0; p = bc_find(s, p + plen, to, pat, plen)) { if (!n) first = p; n++; }
-    return n;
-}
-enum { BC_TWO_SPACERS = 0, BC_N1_SPACER_N2 = 1, BC_FIXED = 2 };   // BcParams::layout
-struct BcParams { char sp1[32], sp2[32]; int layout, lo, hi, bclen, len1, len2, allow_ns, min_q, max_below; double avg_q; };
-
+// One thread per decombined row: the barcode region (R2[:bclength], field 8 of an .n12 row) and its quality string,
+// through bc_row (barcode_core.cuh, where the semantics are written down).  FUZZY false: the exact spacer search only
+// (dcb_barcodes); true: the reference's fuzzy searches too (dcb_barcodes_fuzzy).  A row that needs them (a few percent)
+// runs them inline in its own thread.
+template <bool FUZZY>
 __global__ void __launch_bounds__(128)
 dcb_barcodes_kernel(const unsigned char* __restrict__ bc, const unsigned char* __restrict__ qual, const uint64_t* __restrict__ bc_off,
                     const uint32_t* __restrict__ bc_len, const uint64_t* __restrict__ q_off, const uint32_t* __restrict__ q_len,
-                    uint64_t n, BcParams P, uint8_t* __restrict__ status, uint8_t* __restrict__ n1len, uint64_t* __restrict__ code) {
+                    uint64_t n, BcParams P, uint8_t* __restrict__ status, uint8_t* __restrict__ n1len, uint64_t* __restrict__ code,
+                    uint8_t* __restrict__ match) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const unsigned char* s = bc + bc_off[i];
-    const unsigned char* q = qual + q_off[i];
-    const int L = (int)bc_len[i];
-    status[i] = DCB_BC_HOST; n1len[i] = 0; code[i] = 0;
-    if (L > 250 || (int)q_len[i] != L) return;
-    bool has_n = false, odd = false;
-    for (int p = 0; p < L; p++) {
-        const unsigned char c = s[p];
-        has_n |= c == 'N';
-        odd |= !(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N');
-    }
-    if (has_n && !P.allow_ns) { status[i] = DCB_BC_FAIL_N; return; }                        // collapse.py:388-392
-    if (odd || (P.layout == BC_FIXED && L < P.bclen)) return;
-    int w0, w1;
-    const int hi = L < P.hi ? L : P.hi;
-    const int c1 = bc_count(s, P.lo, hi, P.sp1, P.len1, w0);                                // :405-413
-    if (c1 == 0) return;                                                                    // the fuzzy searches decide
-    if (c1 != 1) { status[i] = DCB_BC_FAIL_NOSPACER; return; }
-    // the barcode symbols (A C G T N S L = 0..6) and their qualities
-    uint64_t cd = (uint64_t)P.bclen << 58;
-    int qsum = 0, qn = 0, below = 0, k = 0;
-    auto sym = [](unsigned char c) -> uint64_t { return c == 'A' ? 0 : c == 'C' ? 1 : c == 'G' ? 2 : c == 'T' ? 3 : 4; };
-    auto addq = [&](int v) { qsum += v; qn++; below += v < P.min_q; };
-    if (P.layout == BC_FIXED) {                                                             // set_barcode: bc[0:bclen], q[0:bclen]
-        for (; k < P.bclen; k++) { cd |= sym(s[k]) << (3 * k); addq((int)q[k] - 33); }
-    } else {
-        int b1s = 0, b1e = w0, b2s = w0 + P.len1;                                           // I8_single: N1, spacer, N2
-        if (P.layout == BC_TWO_SPACERS) {
-            const int c2 = bc_count(s, P.len1, L, P.sp2, P.len2, w1);                       // :417-422
-            if (c2 == 0) return;
-            if (c2 != 1) { status[i] = DCB_BC_FAIL_NOT2; return; }
-            b1s = w0 + P.len1; b1e = w1; b2s = w1 + P.len2;
-        }
-        const int b2e = b2s + 6, n1 = b1e - b1s;
-        if (n1 <= 3) { status[i] = DCB_BC_FAIL_N1SHORT; return; }                           // :241-254
-        if (n1 >= 9) { status[i] = DCB_BC_FAIL_N1LONG; return; }
-        if (b2e > L) { status[i] = DCB_BC_FAIL_N2END; return; }
-        n1len[i] = (uint8_t)n1;
-        // 12 symbols; a long N1 has no pad quality (11 values)
-        const int take1 = n1 > 6 ? 5 : n1;
-        for (int p = 0; p < take1; p++, k++) { cd |= sym(s[b1s + p]) << (3 * k); addq((int)q[b1s + p] - 33); }
-        if (n1 < 6) for (int p = n1; p < 6; p++, k++) { cd |= 5ull << (3 * k); addq('?' - 33); }   // 'S', quality '?'
-        if (n1 > 6) { cd |= 6ull << (3 * k); k++; }                                               // 'L'; "?" * (6 - n1) is empty
-        for (int p = 0; p < 6; p++, k++) { cd |= sym(s[b2s + p]) << (3 * k); addq((int)q[b2s + p] - 33); }
-    }
-    code[i] = cd;
-    const bool bad_q = below > P.max_below || (double)qsum / (double)qn < P.avg_q;            // :350-352
-    status[i] = bad_q ? DCB_BC_FAIL_QUALITY : DCB_BC_OK;
+    const BcRow r = bc_row<FUZZY>(bc + bc_off[i], (int)bc_len[i], qual + q_off[i], (int)q_len[i], P);
+    status[i] = r.status; n1len[i] = r.n1len; code[i] = r.code;
+    if (match) match[i] = r.match;
 }
 
 struct GrowBuf {            // grow-only device buffer kept between calls (dcb_lev_leq is called once per grouping round)
@@ -631,38 +560,41 @@ static int lev_leq_impl(dcb_dist* d, const uint8_t* symbols, const uint64_t* off
     return DCB_OK;
 }
 
+static int barcodes_impl(dcb_dist* d, const char* bc_text, const uint64_t* bc_off, const uint32_t* bc_len, const char* q_text,
+                         const uint64_t* q_off, const uint32_t* q_len, uint64_t n, const dcb_bc_params* prm, uint8_t* status,
+                         uint8_t* n1len, uint64_t* code, bool fuzzy, uint8_t* match);
+
 int dcb_barcodes(dcb_dist* d, const char* bc_text, const uint64_t* bc_off, const uint32_t* bc_len, const char* q_text,
                  const uint64_t* q_off, const uint32_t* q_len, uint64_t n, const dcb_bc_params* prm, uint8_t* status,
                  uint8_t* n1len, uint64_t* code) {
+    return barcodes_impl(d, bc_text, bc_off, bc_len, q_text, q_off, q_len, n, prm, status, n1len, code, false, nullptr);
+}
+int dcb_barcodes_fuzzy(dcb_dist* d, const char* bc_text, const uint64_t* bc_off, const uint32_t* bc_len, const char* q_text,
+                       const uint64_t* q_off, const uint32_t* q_len, uint64_t n, const dcb_bc_params* prm, int fuzzy,
+                       uint8_t* status, uint8_t* n1len, uint64_t* code, uint8_t* match) {
+    if (n && !match) { dcb_set_error("dcb_barcodes_fuzzy: null argument"); return DCB_EINVAL; }
+    return barcodes_impl(d, bc_text, bc_off, bc_len, q_text, q_off, q_len, n, prm, status, n1len, code, fuzzy != 0, match);
+}
+
+static int barcodes_impl(dcb_dist* d, const char* bc_text, const uint64_t* bc_off, const uint32_t* bc_len, const char* q_text,
+                         const uint64_t* q_off, const uint32_t* q_len, uint64_t n, const dcb_bc_params* prm, uint8_t* status,
+                         uint8_t* n1len, uint64_t* code, bool fuzzy, uint8_t* match) {
     if (!d || !prm || (n && (!bc_text || !bc_off || !bc_len || !q_text || !q_off || !q_len || !status || !n1len || !code))) {
         dcb_set_error("dcb_barcodes: null argument");
         return DCB_EINVAL;
     }
     if (n == 0) return DCB_OK;
     BcParams P;
-    std::memset(&P, 0, sizeof(P));
-    // spacers, window of spacer 1 and barcode length per design (collapse.py:172-189, 367-479)
-    const char *sp1, *sp2 = "";
-    switch (prm->oligo) {
-    case DCB_OLIGO_M13:       sp1 = "GTCGTGACTGGGAAAACCCTGG"; sp2 = "GTCGTGAT"; P.layout = BC_TWO_SPACERS; break;
-    case DCB_OLIGO_I8:        sp1 = "GTCGTGAT"; sp2 = "GTCGTGAT"; P.layout = BC_TWO_SPACERS; break;
-    case DCB_OLIGO_I8_SINGLE: sp1 = "ATCACGAC"; P.layout = BC_N1_SPACER_N2; break;
-    case DCB_OLIGO_NEBIO:     sp1 = "TACGGG"; P.layout = BC_FIXED; P.lo = 18; P.hi = 28; P.bclen = 17; break;
-    case DCB_OLIGO_TAKARA:    sp1 = "GTACGGG"; P.layout = BC_FIXED; P.lo = 0; P.hi = 19; P.bclen = 12; break;
-    default: dcb_set_error("dcb_barcodes: oligo %d has no device path (DCB_OLIGO_* are 0..4)", prm->oligo); return DCB_EUNSUPPORTED;
-    }
-    P.len1 = (int)std::strlen(sp1); P.len2 = (int)std::strlen(sp2);
-    if (P.layout != BC_FIXED) { P.lo = 0; P.hi = 10 + P.len1; P.bclen = 12; }
-    std::memcpy(P.sp1, sp1, P.len1); std::memcpy(P.sp2, sp2, P.len2);
-    P.allow_ns = prm->allow_ns; P.min_q = prm->min_q; P.max_below = prm->max_below; P.avg_q = prm->avg_q;
+    if (!bc_params(*prm, P)) { dcb_set_error("dcb_barcodes: oligo %d has no device path (DCB_OLIGO_* are 0..4)", prm->oligo); return DCB_EUNSUPPORTED; }
     CUDA_TRY(cudaSetDevice(d->device));
     cudaStream_t s = d->stream;
     uint64_t bc_bytes = 0, q_bytes = 0;
     for (uint64_t i = 0; i < n; i++) { bc_bytes = std::max<uint64_t>(bc_bytes, bc_off[i] + bc_len[i]); q_bytes = std::max<uint64_t>(q_bytes, q_off[i] + q_len[i]); }
-    DevMem dbc, dq, dbo, dbl, dqo, dql, dst, dn1, dcd;
+    DevMem dbc, dq, dbo, dbl, dqo, dql, dst, dn1, dcd, dmt;
     CUDA_TRY(dbc.alloc(bc_bytes + 16)); CUDA_TRY(dq.alloc(q_bytes + 16));
     CUDA_TRY(dbo.alloc(n * 8)); CUDA_TRY(dbl.alloc(n * 4)); CUDA_TRY(dqo.alloc(n * 8)); CUDA_TRY(dql.alloc(n * 4));
     CUDA_TRY(dst.alloc(n)); CUDA_TRY(dn1.alloc(n)); CUDA_TRY(dcd.alloc(n * 8));
+    if (match) CUDA_TRY(dmt.alloc(n));
     CUDA_TRY(cudaMemcpyAsync(dbc.p, bc_text, bc_bytes, cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(dq.p, q_text, q_bytes, cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(dbo.p, bc_off, n * 8, cudaMemcpyHostToDevice, s));
@@ -672,14 +604,21 @@ int dcb_barcodes(dcb_dist* d, const char* bc_text, const uint64_t* bc_off, const
     Events ev;
     CUDA_TRY(cudaEventCreate(&ev.a)); CUDA_TRY(cudaEventCreate(&ev.b));
     CUDA_TRY(cudaEventRecord(ev.a, s));
-    dcb_barcodes_kernel<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(dbc.as<unsigned char>(), dq.as<unsigned char>(), dbo.as<uint64_t>(),
-                                                                   dbl.as<uint32_t>(), dqo.as<uint64_t>(), dql.as<uint32_t>(), n, P,
-                                                                   dst.as<uint8_t>(), dn1.as<uint8_t>(), dcd.as<uint64_t>());
+    const unsigned blocks = (unsigned)((n + 127) / 128);
+    if (match)        // dcb_barcodes_fuzzy, either way of the switch
+        (fuzzy ? dcb_barcodes_kernel<true> : dcb_barcodes_kernel<false>)<<<blocks, 128, 0, s>>>(
+            dbc.as<unsigned char>(), dq.as<unsigned char>(), dbo.as<uint64_t>(), dbl.as<uint32_t>(), dqo.as<uint64_t>(),
+            dql.as<uint32_t>(), n, P, dst.as<uint8_t>(), dn1.as<uint8_t>(), dcd.as<uint64_t>(), dmt.as<uint8_t>());
+    else
+        dcb_barcodes_kernel<false><<<blocks, 128, 0, s>>>(dbc.as<unsigned char>(), dq.as<unsigned char>(), dbo.as<uint64_t>(),
+                                                          dbl.as<uint32_t>(), dqo.as<uint64_t>(), dql.as<uint32_t>(), n, P,
+                                                          dst.as<uint8_t>(), dn1.as<uint8_t>(), dcd.as<uint64_t>(), nullptr);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaEventRecord(ev.b, s));
     CUDA_TRY(cudaMemcpyAsync(status, dst.p, n, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaMemcpyAsync(n1len, dn1.p, n, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaMemcpyAsync(code, dcd.p, n * 8, cudaMemcpyDeviceToHost, s));
+    if (match) CUDA_TRY(cudaMemcpyAsync(match, dmt.p, n, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, ev.a, ev.b) == cudaSuccess) d->last_ms = ms;

@@ -368,6 +368,18 @@ typedef struct dcb_bc_params {
 int dcb_barcodes(dcb_dist*, const char* bc_text, const uint64_t* bc_off, const uint32_t* bc_len, const char* q_text,
                  const uint64_t* q_off, const uint32_t* q_len, uint64_t n, const dcb_bc_params* prm, uint8_t* status,
                  uint8_t* n1len, uint64_t* code);
+/* dcb_barcodes with the reference's fuzzy spacer searches (spacerSearch, collapse.py:205-213: an exact findall, else
+ * {1s<=2}, else {2i+2d+1s<=2}) on the device when fuzzy != 0; fuzzy == 0 gives what dcb_barcodes gives.  With fuzzy on,
+ * DCB_BC_HOST is left only for a symbol outside ACGTN, a quality string of another length, a region longer than 250 and
+ * (TAKARA) a region shorter than 12; a row whose spacers no stage finds once is DCB_BC_FAIL_NOSPACER / _NOT2.  Also per row:
+ *   match   for DCB_BC_OK and DCB_BC_FAIL_QUALITY rows: 0 = both spacers found as in the oligo, 1 = a fuzzy search placed
+ *           either of them (0 on every other row).  The caller derives the reference's match counters from it and n1len:
+ *           getbarcode_pass_exactmatch (match 0) or _regexmatch (match 1); with match 1 getbarcode_pass_fuzzymatch_rightlen
+ *           (N1 of 6; every NEBIO / TAKARA row), _short (N1 of 4-5) or _long (N1 of 7-8); with match 0 and N1 of 6 (every
+ *           NEBIO / TAKARA row) getbarcode_pass_other. */
+int dcb_barcodes_fuzzy(dcb_dist*, const char* bc_text, const uint64_t* bc_off, const uint32_t* bc_len, const char* q_text,
+                       const uint64_t* q_off, const uint32_t* q_len, uint64_t n, const dcb_bc_params* prm, int fuzzy,
+                       uint8_t* status, uint8_t* n1len, uint64_t* code, uint8_t* match);
 
 /* ---------------------------------------------------------------------------------------------
  * Translate stage: get_cdr3 (translate.py:257-357) for DCR rows and the AIRR .tsv line of each, as

@@ -5,8 +5,10 @@ dcb_barcodes for each ligation-oligo design on 42-nt barcode regions (the genera
 re-laid out per design by tests/oligo_layouts.py).
 
     python tools/bench_collapse.py [--umis 200000] [--pairs 2000000] [--barcode-rows 10000000]     (GPU box)
+    python tools/bench_collapse.py --fuzzy-rows 1000000                                           (GPU box)
 
-Prints one JSON line; device times come from the library's own CUDA events (dcb_dist_last_ms)."""
+Prints one JSON line; device times come from the library's own CUDA events (dcb_dist_last_ms).  --fuzzy-rows measures
+only the fuzzy spacer searches of dcb_barcodes_fuzzy (bench_fuzzy)."""
 import argparse
 import json
 import os
@@ -26,7 +28,11 @@ def main():
     ap.add_argument("--pairs", type=int, default=2_000_000)
     ap.add_argument("--big", type=int, default=2_000_000, help="UMIs of the configs[3]-scale pair search (0 = skip)")
     ap.add_argument("--barcode-rows", type=int, default=10_000_000, help="barcode regions per design for dcb_barcodes (0 = skip)")
+    ap.add_argument("--fuzzy-rows", type=int, default=0, help="only bench_fuzzy, over this many barcode regions per design and rate")
     args = ap.parse_args()
+    if args.fuzzy_rows:
+        print(json.dumps(bench_fuzzy(args.fuzzy_rows)))
+        return
     from decombinator_b200 import _lib
     rng = np.random.default_rng(20260004)
     U = args.umis
@@ -114,6 +120,89 @@ def bench_barcodes(d, n):
         ms = d.last_ms()
         out[oligo] = {"device_ms": ms, "rows_per_s": n / (ms / 1e3), "decided_on_device": float((st != _lib.BC_HOST).mean()),
                       "passed": float((st == _lib.BC_OK).mean())}
+    return out
+
+
+def _indels(a, rng, rate, span=42):
+    """Each of the first `span` bases of every row of a (uint8, rows x width) deleted (a random base appended) or followed by
+    an inserted base (the last base dropped) with probability `rate`."""
+    k = rng.binomial(span, rate, size=len(a))
+    for i in np.nonzero(k)[0].tolist():
+        row = a[i].tolist()
+        for _ in range(int(k[i])):
+            p = int(rng.integers(span))
+            if rng.random() < 0.5:
+                row = row[:p] + row[p + 1:] + [int(rng.choice(list(b"ACGT")))]
+            else:
+                row = row[:p] + [int(rng.choice(list(b"ACGT")))] + row[p:-1]
+        a[i] = row
+    return a
+
+
+def bench_fuzzy(n):
+    """Per design and read-2 substitution rate (0.5, 1 and 2 %, plus 0.1 % indels per base of the 42-nt region): the rows
+    dcb_barcodes hands back (exact spacer searches only) and dcb_barcodes_fuzzy hands back, the kernel time of each (CUDA
+    events, best of three, the quality text one cached row), and the wall time of collapse._filter_rows over the same
+    regions as the columns of an .n12 file (the `collapse` command's path) with DCB_BC_FUZZY=0 and with the default,
+    alternated, with the kept rows and counters compared."""
+    import tempfile
+    import oligo_layouts
+    from decombinator_b200 import _lib, collapse, tags
+    info = tags.load("human", "extended", "b")
+    rng = np.random.default_rng(20261022)
+    d = _lib.Dist(0)
+    bo = np.arange(n, dtype=np.uint64) * np.uint64(62)
+    bl = np.full(n, 42, dtype=np.uint32)
+    qbuf, qo = np.full(64, ord("I"), dtype=np.uint8), np.zeros(n, dtype=np.uint64)
+    out = {"rows": n, "region": "42 nt of a 62-nt read 2, substitutions at the rate given + 0.1 % indels per base", "runs": []}
+    seqs = np.frombuffer(b"ACGT", dtype=np.uint8)[rng.integers(0, 4, size=(n, 30))]
+    head = np.frombuffer(b"".join(b"12, 3, 1, 2, ACGT, SYN:%07d, " % i for i in range(n)), dtype=np.uint8).reshape(n, -1)
+    comma = np.frombuffer(b", ", dtype=np.uint8)
+    tmp = tempfile.mkdtemp()
+    for rate in (0.005, 0.01, 0.02):
+        syn = _lib.Synth([(info.v_regions, info.j_regions)], 20260004, 250, 62, 0.0, 0.0, 0.0, umi_pool=max(1000, n // 50),
+                         sub_rate2=rate)
+        r2 = syn.reads(0, n, want_r2=True)[1].reshape(n, 62)
+        for oligo in ("M13", "I8", "I8_single", "NEBIO", "TAKARA"):
+            reg = np.ascontiguousarray(r2 if oligo == "M13" else oligo_layouts.relayout_array(r2, oligo))
+            reg = _indels(reg, rng, 0.001)
+            text = reg.reshape(-1)
+            code = _lib.OLIGOS_ON_DEVICE[oligo.lower()]
+            d.barcodes_arrays(text, bo[:1000], bl[:1000], qbuf, qo[:1000], bl[:1000], code, False, 20, 1, 30)
+            d.barcodes_arrays(text, bo[:1000], bl[:1000], qbuf, qo[:1000], bl[:1000], code, False, 20, 1, 30, True)
+            ms_off, ms_on = [], []
+            for _ in range(3):
+                st_off = d.barcodes_arrays(text, bo, bl, qbuf, qo, bl, code, False, 20, 1, 30)[0]
+                ms_off.append(d.last_ms())
+                st_on, _, _, match = d.barcodes_arrays(text, bo, bl, qbuf, qo, bl, code, False, 20, 1, 30, True)
+                ms_on.append(d.last_ms())
+            # the same regions as an .n12 file: what collapse reads, timed through _filter_rows
+            q = np.full((n, 30), ord("I"), dtype=np.uint8)
+            rows = np.concatenate([head, seqs, np.tile(comma, (n, 1)), q, np.tile(comma, (n, 1)), reg[:, :42], np.tile(comma, (n, 1)),
+                                   np.full((n, 42), ord("I"), dtype=np.uint8), np.full((n, 1), ord("\n"), dtype=np.uint8)], axis=1)
+            path = os.path.join(tmp, "rows.n12")
+            rows.tofile(path)
+            n12 = collapse.N12Columns.from_file(path, open)
+            args = {"oligo": oligo, "sampling_analysis": False, "allowNs": False, "lenthreshold": 130}
+            wall = {"0": [], "1": []}
+            result = {}
+            for _ in range(2):
+                for mode in ("0", "1"):
+                    os.environ["DCB_BC_FUZZY"] = mode
+                    collapse.counts = collapse.coll.Counter()
+                    t0 = time.perf_counter()
+                    kept, dcrs, _ = collapse._filter_rows(n12, args, [20, 1, 30], True, False)
+                    wall[mode].append(round(time.perf_counter() - t0, 3))
+                    result[mode] = (kept, dcrs, {k: v for k, v in collapse.counts.items() if isinstance(v, int)})
+            del os.environ["DCB_BC_FUZZY"]
+            placed = (st_on == _lib.BC_OK) | (st_on == _lib.BC_FAIL_QUALITY)
+            out["runs"].append({
+                "oligo": oligo, "sub_rate2": rate, "handed_back_exact_only": float((st_off == _lib.BC_HOST).mean()),
+                "handed_back_fuzzy": float((st_on == _lib.BC_HOST).mean()), "placed_by_fuzzy_text": float((placed & (match != 0)).mean()),
+                "kernel_ms_exact_only": min(ms_off), "kernel_ms_fuzzy": min(ms_on),
+                "filter_rows_s_DCB_BC_FUZZY_0": wall["0"], "filter_rows_s_default": wall["1"],
+                "filter_rows_same_output": result["0"] == result["1"]})
+            print(json.dumps(out["runs"][-1]), file=sys.stderr, flush=True)
     return out
 
 

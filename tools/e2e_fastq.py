@@ -3,6 +3,7 @@
 
     python tools/e2e_fastq.py [--reads 2000000] [--python-fastq]
     python tools/e2e_fastq.py --pipeline [--oligo I8_single|NEBIO|TAKARA] [--cli]
+    python tools/e2e_fastq.py --pipeline --fuzzy-ab [--oligo ...] [--sub2 0.01]
 
 Writes R1/R2 files of the configs[1] recipe under /tmp, runs the drop-in stage function (decombine.py:881 of the
 reference) and prints where the wall time goes: ingest (FASTQ text -> record index), pack, device, row assembly.  With --pipeline --oligo, read 2 is re-laid out for that ligation-oligo design
@@ -10,6 +11,8 @@ reference) and prints where the wall time goes: ingest (FASTQ text -> record ind
 host (the device path restricted to M13 and I8 in this process, as before the device took the other designs).  With
 --pipeline --cli, `pipeline` runs as the command line runs it (the .n12, .freq and .tsv written with -dz, the translate
 stage handing its text to the writer), twice with the translate stage on the device and twice on the host, alternated.
+With --pipeline --fuzzy-ab, read 2 gets --sub2 substitutions and 0.1 % indels per base of its barcode region, and
+`pipeline` runs twice with DCB_BC_FUZZY=0 (the fuzzy spacer searches on the host) and twice as shipped, alternated.
 """
 import argparse
 import json
@@ -35,16 +38,22 @@ def main():
     ap.add_argument("--oligo", default="M13", choices=["M13", "I8", "I8_single", "NEBIO", "TAKARA"],
                     help="with --pipeline: read 2 laid out for this ligation-oligo design")
     ap.add_argument("--cli", action="store_true", help="with --pipeline: the command line's path, translate on the device and on the host")
+    ap.add_argument("--fuzzy-ab", action="store_true", help="with --pipeline: DCB_BC_FUZZY=0 against the default, alternated")
+    ap.add_argument("--sub2", type=float, default=0.0, help="substitution rate of read 2")
     args = ap.parse_args()
     from decombinator_b200 import _lib, decombine, fastq, io, tags
     info = tags.load("human", "extended", "b")
     L, n = 250, args.reads
     syn = _lib.Synth([(info.v_regions, info.j_regions)], 20260002, L, 42 + 20, 0.0, 0.0, 0.0,
-                     umi_pool=(max(1000, n // 20) if args.pipeline else 0))
+                     umi_pool=(max(1000, n // 20) if args.pipeline else 0), sub_rate2=args.sub2)
     r1, r2 = syn.reads(0, n, want_r2=True)
     if args.oligo != "M13":
         import oligo_layouts
         r2 = oligo_layouts.relayout_array(r2.reshape(n, 62), args.oligo).reshape(-1)
+    if args.fuzzy_ab:
+        sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+        from bench_collapse import _indels
+        r2 = _indels(np.ascontiguousarray(r2.reshape(n, 62)), np.random.default_rng(20261022), 0.001).reshape(-1)
     os.makedirs("/tmp/e2e", exist_ok=True)
     p1, p2 = "/tmp/e2e/syn_1.fq", "/tmp/e2e/syn_2.fq"
     t0 = time.perf_counter()
@@ -78,6 +87,21 @@ def main():
         t0 = time.perf_counter()
         rows = decombine.decombinator(dict(ia))
         t_dec = time.perf_counter() - t0
+        if args.fuzzy_ab:
+            from decombinator_b200 import collapse
+            times, outs = {"0": [], "1": []}, {}
+            for rep in range(2):
+                for mode in ("0", "1"):
+                    os.environ["DCB_BC_FUZZY"] = mode
+                    t0 = time.perf_counter()
+                    out = pipeline.run(dict(ia))
+                    times[mode].append(round(time.perf_counter() - t0, 2))
+                    outs[mode] = (out, {k: v for k, v in collapse.counts.items() if isinstance(v, int) and not k.startswith("time_")})
+            same = outs["0"][0].equals(outs["1"][0]) and outs["0"][1] == outs["1"][1]
+            print(json.dumps({"reads": n, "oligo": args.oligo, "sub2": args.sub2, "indels_per_base": 0.001,
+                              "pipeline_s_DCB_BC_FUZZY_0": times["0"], "pipeline_s_default": times["1"],
+                              "regexmatch": outs["1"][1].get("getbarcode_pass_regexmatch", 0), "same_output": bool(same)}))
+            return
         if args.cli:
             import hashlib
             from decombinator_b200 import translate
