@@ -105,6 +105,15 @@ def lib():
     pu64 = ctypes.POINTER(u64)
     L.dcb_bgzf_inflate.argtypes = [vp, vp, vp, vp, vp, u64, vp, i32]
     L.dcb_bgzf_inflate.restype = ctypes.c_int
+    L.dcb_inflate_create.argtypes = [i32, vp, u64, u64, u64, ctypes.POINTER(ctypes.c_void_p)]
+    L.dcb_inflate_find_starts.argtypes = [vp, vp, u64, pu64]
+    L.dcb_inflate_begin.argtypes = [vp, vp, u64]
+    L.dcb_inflate_begin_members.argtypes = [vp, vp, vp, vp, u64]
+    L.dcb_inflate_read.argtypes = [vp, vp, u64, pu64, pu64]
+    L.dcb_inflate_destroy.argtypes = [vp]
+    L.dcb_inflate_destroy.restype = None
+    for f in (L.dcb_inflate_create, L.dcb_inflate_find_starts, L.dcb_inflate_begin, L.dcb_inflate_begin_members, L.dcb_inflate_read):
+        f.restype = ctypes.c_int
     L.dcb_group_create.argtypes = [vp, u64, u64, vp, vp, ctypes.POINTER(ctypes.c_void_p)]
     L.dcb_group_step.argtypes = [vp, pu64]
     L.dcb_group_pairs.argtypes = [vp, pu64, pu64, vp, vp, vp, vp, vp, ctypes.POINTER(ctypes.c_int)]
@@ -416,6 +425,67 @@ def n12_collapse_rows(text, off, ln, keep, n_threads=None):
     if nrows.value == 0xFFFFFFFFFFFFFFFF:
         return None
     return NativeText(out.value, nbytes.value), int(nrows.value)
+
+
+NO_START = 2 ** 64 - 1        # dcb_inflate_find_starts: no candidate in this chunk
+
+
+def _inflate_check(rc, what):
+    if rc != 0:
+        err = DcbError("%s failed (%d): %s" % (what, rc, lib().dcb_last_error().decode()))
+        err.rc = rc
+        raise err
+
+
+def gpu_inflate(raw, device=0, members=None, chunk_bytes=0, segment_bytes=0, starts_hook=None):
+    """A gzip file inflated on the GPU (dcb_inflate_*) into an anonymous memory map; b"" when it holds no bytes.
+
+    raw: the compressed file (bytes-like).  members: [(start, end, isize), ...] of a BGZF file (fastq._bgzf_blocks), else
+    the file is decoded as one stream from the candidate starts of dcb_inflate_find_starts, passed through starts_hook
+    (tests) when given.  Raises DcbError with .rc = -2 (DCB_ENOGPU) without a device, -5 (DCB_EIO) for a damaged file."""
+    import mmap
+    L = lib()
+    src = np.frombuffer(raw, dtype=np.uint8)
+    h = ctypes.c_void_p()
+    _inflate_check(L.dcb_inflate_create(int(device), src.ctypes.data if len(src) else None, len(src), int(chunk_bytes), int(segment_bytes),
+                                        ctypes.byref(h)), "dcb_inflate_create")
+    try:
+        if members is not None:
+            arr = np.array(members, dtype=np.uint64).reshape(-1, 3)
+            start, end, isize = (np.ascontiguousarray(arr[:, i]) for i in range(3))
+            isize = isize.astype(np.uint32)
+            _inflate_check(L.dcb_inflate_begin_members(h, start.ctypes.data, end.ctypes.data, isize.ctypes.data, len(arr)),
+                           "dcb_inflate_begin_members")
+            cap = int(arr[:, 2].sum())
+        else:
+            n = ctypes.c_uint64()
+            _inflate_check(L.dcb_inflate_find_starts(h, None, 0, ctypes.byref(n)), "dcb_inflate_find_starts")
+            starts = np.zeros(max(1, n.value), dtype=np.uint64)
+            _inflate_check(L.dcb_inflate_find_starts(h, starts.ctypes.data, len(starts), ctypes.byref(n)), "dcb_inflate_find_starts")
+            if starts_hook is not None:
+                starts = np.ascontiguousarray(starts_hook(starts.copy()), dtype=np.uint64)
+            _inflate_check(L.dcb_inflate_begin(h, starts.ctypes.data, len(starts)), "dcb_inflate_begin")
+            cap = 4 * len(src)
+        cap = max(cap, 1 << 20)
+        out = mmap.mmap(-1, cap, flags=mmap.MAP_PRIVATE | mmap.MAP_ANONYMOUS)
+        pos = 0
+        got, more = ctypes.c_uint64(), ctypes.c_uint64()
+        while True:
+            view = ctypes.c_char.from_buffer(out)
+            addr = ctypes.addressof(view)
+            del view                                   # (an exported buffer would keep the map from growing)
+            _inflate_check(L.dcb_inflate_read(h, addr + pos, cap - pos, ctypes.byref(got), ctypes.byref(more)), "dcb_inflate_read")
+            pos += got.value
+            if not more.value:
+                break
+            cap = max(2 * cap, pos + more.value)
+            out.resize(cap)
+    finally:
+        L.dcb_inflate_destroy(h)
+    if pos == 0:
+        return b""
+    out.resize(pos)
+    return out
 
 
 def bgzf_inflate(raw, start, end, isize, out_off, out, n_threads=None):

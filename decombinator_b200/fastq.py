@@ -204,10 +204,35 @@ def _bgzf_blocks(raw):
     return blocks or None
 
 
+# BGZF files are inflated by the host threads: on the B200 box they beat one GPU decoder per 64 KB member (DESIGN §6).
+BGZF_ON_DEVICE = False
+# A single stream goes to the GPU unless its text is more than this many times the file's size (ISIZE of the last member
+# over the file size).  One decoder thread per chunk writes its text serially, and highly compressible files have few
+# chunks for a lot of text: on the B200 box the device inflated FASTQ of 6.5:1 at 2.8x the host's rate, and was slower
+# than the host on synthetic FASTQ of 15:1 and 9:1 (constant quality strings) (DESIGN §6).
+DEVICE_MAX_RATIO = 8
+
+
+def _device_gunzip(raw, blocks):
+    """The file inflated on the GPU (LOCAL_RANK selects it), or None: no usable device, a BGZF file (see BGZF_ON_DEVICE), or
+    any failure of the device path -- a damaged file then reaches the host path, which raises what it raises today."""
+    if blocks and not BGZF_ON_DEVICE:
+        return None
+    if not blocks and len(raw) >= 18 and int.from_bytes(raw[-4:], "little") > DEVICE_MAX_RATIO * len(raw):
+        return None
+    from . import _lib
+    try:
+        return _lib.gpu_inflate(raw, device=int(os.environ.get("LOCAL_RANK", "0")), members=blocks)
+    except _lib.DcbError:
+        return None
+
+
 def gunzip_file(path, n_threads=None):
     """The decompressed bytes of a .gz file in an anonymous memory map (the same kind of object a plain file is read
-    through).  A BGZF file is inflated block by block on all host threads (dcb_bgzf_inflate); any other gzip file --
-    one member or several -- is one deflate stream after the other, inflated in slices straight into the map."""
+    through).  A single stream or a chain of members is inflated on the GPU when one is usable (dcb_inflate_*, csrc/inflate.cu).
+    Otherwise, and whenever the device path reports anything but success: a BGZF file is inflated block by block on all host
+    threads (dcb_bgzf_inflate); any other gzip file -- one member or several -- is one deflate stream after the other,
+    inflated in slices straight into the map."""
     with open(path, "rb") as fh:
         try:
             raw = mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ)
@@ -216,6 +241,9 @@ def gunzip_file(path, n_threads=None):
     if len(raw) == 0:
         return b""
     blocks = _bgzf_blocks(raw)
+    out = _device_gunzip(raw, blocks)
+    if out is not None:
+        return out
     if blocks:
         from . import _lib
         arr = np.array(blocks, dtype=np.uint64)

@@ -202,6 +202,34 @@ void dcb_buffer_free(char*);
 int dcb_bgzf_inflate(const unsigned char* raw, const uint64_t* start, const uint64_t* end, const uint32_t* isize, const uint64_t* out_off,
                      uint64_t n_blocks, unsigned char* out, int n_threads);
 
+/* Compressed FASTQ inflated on the GPU (csrc/inflate.cu).  One handle per file; it owns its device buffers and stream.
+ *   dcb_inflate_create         copies the gzip file (n_bytes of gz, which must stay valid until destroy) to the device.
+ *                              chunk_bytes: nominal chunk of the start finder (0: 64 KiB; at least 1 KiB);
+ *                              segment_bytes: compressed bytes processed per segment (0: 1 GiB).  DCB_ENOGPU without a device.
+ *   One deflate stream, or gzip members without sizes:
+ *     dcb_inflate_find_starts  one candidate start per nominal chunk: the bit offset of the first dynamic block header with
+ *                              complete codes at or after the chunk's first byte, UINT64_MAX when there is none; entry 0 is
+ *                              the first block of the file.  starts == NULL: *n_chunks only.
+ *     dcb_inflate_begin        decode from these starts (ascending, UINT64_MAX entries skipped, the first one the file's
+ *                              first block).  Any list is safe: only starts that a chain of decodes from the first one lands
+ *                              on are kept, so a wrong candidate costs time, never output.
+ *   Members with known bounds (BGZF): dcb_inflate_begin_members with each member's raw deflate data gz[start[k], end[k])
+ *   and its ISIZE, the CRC-32 behind it (empty members left out).
+ *   dcb_inflate_read           writes the inflated bytes, whole segments at a time, to out (cap bytes) and sets *produced.
+ *                              *more == 0: everything is written.  Otherwise the next segment does not fit: it stays decoded
+ *                              on the device and *more is its size; call again with a buffer of at least that many bytes
+ *                              (out advanced past what was written).  A stream's size is not known before it is decoded
+ *                              (ISIZE holds it modulo 2^32), so the caller grows its buffer between calls and nothing is
+ *                              decoded twice.  DCB_EIO: the file is damaged (invalid data, a chain chunk at its bit limit,
+ *                              a CRC-32 or ISIZE mismatch); the text says which. */
+typedef struct dcb_inflate dcb_inflate;
+int dcb_inflate_create(int device, const unsigned char* gz, uint64_t n_bytes, uint64_t chunk_bytes, uint64_t segment_bytes, dcb_inflate** out);
+int dcb_inflate_find_starts(dcb_inflate*, uint64_t* starts, uint64_t cap, uint64_t* n_chunks);
+int dcb_inflate_begin(dcb_inflate*, const uint64_t* starts, uint64_t n);
+int dcb_inflate_begin_members(dcb_inflate*, const uint64_t* start, const uint64_t* end, const uint32_t* isize, uint64_t n);
+int dcb_inflate_read(dcb_inflate*, unsigned char* out, uint64_t cap, uint64_t* produced, uint64_t* more);
+void dcb_inflate_destroy(dcb_inflate*);
+
 /* The order-dependent grouping of collapse's read_in_data (collapse.py:595-682) over columns instead of a Python loop over
  * rows: per barcode, rows in input order found / join / kill the barcode's group (rules: csrc/group.cpp).  Host logic; the
  * sequence comparisons it needs (are_seqs_equivalent, collapse.py:355-360) are the caller's to fetch from the GPU:

@@ -32,6 +32,7 @@ def main():
     ap.add_argument("--reads", type=int, default=2_000_000)
     ap.add_argument("--python-fastq", action="store_true", help="use the general (Python) parser instead of the native index")
     ap.add_argument("--gz", choices=["gzip", "bgzf"], default=None, help="compress the two files first: one gzip stream each, or BGZF blocks")
+    ap.add_argument("--host-inflate", action="store_true", help="with --gz: inflate on the host as without a GPU (the path before dcb_inflate)")
     ap.add_argument("--rows-as-text", action="store_true", help="what the `decombine` command does: rows handed over as .n12 text")
     ap.add_argument("--profile", action="store_true", help="cProfile of the timed decombinator() call")
     ap.add_argument("--pipeline", action="store_true", help="decombine + collapse (pipeline.run) on reads with repeated UMIs")
@@ -42,6 +43,8 @@ def main():
     ap.add_argument("--sub2", type=float, default=0.0, help="substitution rate of read 2")
     args = ap.parse_args()
     from decombinator_b200 import _lib, decombine, fastq, io, tags
+    if args.host_inflate:
+        fastq._device_gunzip = lambda raw, blocks: None
     info = tags.load("human", "extended", "b")
     L, n = 250, args.reads
     syn = _lib.Synth([(info.v_regions, info.j_regions)], 20260002, L, 42 + 20, 0.0, 0.0, 0.0,
@@ -163,7 +166,7 @@ def main():
     if args.profile:
         pr.disable()
         pstats.Stats(pr).sort_stats("cumulative").print_stats(22)
-    print(json.dumps({"reads": n, "parser": "python" if args.python_fastq else "native", "rows_as_text": bool(args.rows_as_text), "fastq_write_s": round(t_write, 2),
+    print(json.dumps({"reads": n, "gz": args.gz, "host_inflate": bool(args.host_inflate), "parser": "python" if args.python_fastq else "native", "rows_as_text": bool(args.rows_as_text), "fastq_write_s": round(t_write, 2),
                       "ingest_only_s": round(t_ingest, 3), "decombinator_s": round(t_total, 2), "rows": len(rows),
                       "reads_per_s": round(n / t_total), "ingest_reads_per_s": round(n / t_ingest)}))
 
